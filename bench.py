@@ -1,8 +1,11 @@
 #!/usr/bin/env python
 """bench.py — images/sec of the denoise + decode hot path (BASELINE.json metric).
 
-  python bench.py --gpus N --steps K --warmup W [--impl ours|reference] [--workload C4|C2|C3]
+  python bench.py --gpus N --steps K --warmup W [--impl ours|reference] [--workload C4|C2|C3] [--dump-outputs DIR]
   (N > 1: launched by torchrun, one rank per GPU; batch sharded by image, no per-step collective.)
+
+--dump-outputs DIR writes what the last timed step returned (rank 0's shard) as DIR/<name>.npy, float32; the inputs are
+seeded, so two builds run with the same arguments can be compared output for output (see dump_outputs).
 
 A "step" = one batch of images through the whole hot path (sample_euler over all denoise steps + VAE decode).
 Default workload C4: FLUX.1-schnell, 1024x1024 (latent 128x128), 4 steps, cfg 0, batch 4 images per GPU
@@ -97,6 +100,27 @@ def vae_roofline(decode_ms, images, lat, peaks):
             "dram_gbs": gb / (ms_img * 1e-3), "hbm_frac": gb / (ms_img * 1e-3) / peaks["hbm_gbs"],
             "dram_source": "profiles/r02_vae_dram_B{1,4}_norm1.txt (ncu dram__bytes_read+write of one decode)",
             "bound": "tensor (3x3 convs at ~780 FLOP/B); the HBM-bound kernels are listed in DESIGN.md §5"}
+
+
+DUMP_BYTES = 60 << 20      # all dumped arrays together stay under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each array as out_dir/<name>.npy in float32.  An array larger than its equal share of DUMP_BYTES is cut to
+    a fixed sample: the elements at np.sort(np.random.RandomState(0).choice(numel, k, replace=False)) of the flattened
+    array, written flat as <name>_sample.npy, so arrays of the same shape are sampled at the same positions in every
+    run.  Returns {file name: shape written}."""
+    os.makedirs(out_dir, exist_ok=True)
+    cap = DUMP_BYTES // max(len(arrays), 1) // 4
+    written = {}
+    for name, t in arrays.items():
+        a = t.detach().to(device="cpu", dtype=torch.float32).numpy()
+        if a.size > cap:
+            idx = np.sort(np.random.RandomState(0).choice(a.size, cap, replace=False))
+            a, name = a.reshape(-1)[idx], name + "_sample"
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
+        written[name + ".npy"] = list(a.shape)
+    return written
 
 
 def load_peaks():
@@ -291,10 +315,10 @@ def run_ours(args):
                                          latent_size=(lat, lat), seed=seeds, noise=noise_dev)
         ev[1].record()
         lat16 = ops.cast_to_16(latent, pipe.activation_dtype)
-        out = pipe._decode(lat16, want_u8=True)
+        images, images_u8 = pipe._decode(lat16, want_u8=True)
         ev[2].record()
         split["ev"] = ev
-        return out
+        return {"latents": latent, "images": images, "images_uint8": images_u8}
 
     def step_e2e():
         imgs, log = pipe.generate_image("", num_steps=steps, cfg_weight=cfgw, latent_size=(lat, lat), seed=seeds,
@@ -318,12 +342,16 @@ def run_ours(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        step_device()
+        last = step_device()
     e1.record()
     torch.cuda.synchronize()
     barrier()
     launches = ops.launch_count() - launches0
     clk = clocks.stop()
+    if args.dump_outputs and rank == 0:        # before anything else runs on the buffers the last step returned
+        dumped = dump_outputs(args.dump_outputs, last)
+        print(f"bench: wrote {dumped} to {args.dump_outputs}", file=sys.stderr, flush=True)
+    del last
     split["denoise"] = split["ev"][0].elapsed_time(split["ev"][1])
     split["decode"] = split["ev"][1].elapsed_time(split["ev"][2])
     t_mine = e0.elapsed_time(e1) / 1e3
@@ -466,7 +494,11 @@ def main():
     ap.add_argument("--workload", default="C4", choices=sorted(WORKLOADS))
     ap.add_argument("--images-per-gpu", type=int, default=0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

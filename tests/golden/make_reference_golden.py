@@ -1,11 +1,12 @@
 """Golden vectors from the REFERENCE'S OWN PyTorch modules (python/src/diffusionkit/torch/mmdit.py, vae.py), run in
-this container from /root/reference with the stand-ins of tests/golden/reference_shims.py for the four argmaxtools
+plain PyTorch from a reference checkout ($DIFFUSIONKIT_REFERENCE) with the stand-ins of tests/golden/reference_shims.py for the four argmaxtools
 building blocks they import.  Writes tests/golden/reference_torch_mmdit.npz and reference_torch_vae_decoder.npz.
 
 The weights are not stored: they are the deterministic initialiser of diffusionkit_b200/weights.py (seeds below),
 converted into the reference modules' state_dict layout here and loaded with strict=True.
 
-Run from the repo root (needs /root/reference):  python tests/golden/make_reference_golden.py
+Run from the repo root:
+    DIFFUSIONKIT_REFERENCE=<argmaxinc/DiffusionKit checkout> python tests/golden/make_reference_golden.py
 """
 import os
 import sys
@@ -109,7 +110,7 @@ def make_inputs():
 
 
 if __name__ == "__main__":
-    assert rs.reference_available(), "needs /root/reference"
+    assert rs.reference_available(), "set DIFFUSIONKIT_REFERENCE to an argmaxinc/DiffusionKit checkout"
     latent, text, pooled, timestep, z = make_inputs()
     y = run_reference_mmdit(latent, text, pooled, timestep)
     np.savez_compressed(os.path.join(HERE, "reference_torch_mmdit.npz"), latent=latent.numpy(), text=text.numpy(),

@@ -1,11 +1,12 @@
 """Golden vectors from the reference's MLX SOURCE files (python/src/diffusionkit/mlx/mmdit.py, config.py, sampler.py,
-vae.py), imported from /root/reference and executed on tests/golden/mlx_standin.py — a torch-backed stand-in for the MLX
-primitives they call (MLX itself cannot run in this container).  This pins the oracle's wiring of the FLUX path (single-
+vae.py), imported from a reference checkout ($DIFFUSIONKIT_REFERENCE) and executed on tests/golden/mlx_standin.py — a torch-backed stand-in for the MLX
+primitives they call (MLX itself runs on Apple silicon only).  This pins the oracle's wiring of the FLUX path (single-
 stream blocks, RoPE, QK-RMSNorm, reshape-patchify, [text | image] order, modulation cache) and of the SD3 path against
 the reference's own code; the fixtures are fp32.
 
 Writes tests/golden/reference_mlxsrc_{flux,sd3}_mmdit.npz, reference_mlxsrc_vae.npz, reference_mlxsrc_sampler.json.
-Run from the repo root (needs /root/reference):  python tests/golden/make_reference_mlx_golden.py
+Run from the repo root:
+    DIFFUSIONKIT_REFERENCE=<argmaxinc/DiffusionKit checkout> python tests/golden/make_reference_mlx_golden.py
 """
 import importlib
 import json
@@ -19,7 +20,6 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF_MLX_DIR = "/root/reference/python/src/diffusionkit/mlx"
 
 from diffusionkit_b200.config import (PositionalEncoding, VAEDecoderConfig, VAEEncoderConfig,  # noqa: E402
                                       tiny_flux_config, tiny_sd3_config)
@@ -27,15 +27,17 @@ from diffusionkit_b200.weights import (init_params, mmdit_param_specs, vae_decod
                                        vae_encoder_param_specs)
 from tests.golden import mlx_standin, reference_shims  # noqa: E402
 
+REF_MLX_DIR = os.path.join(reference_shims.REFERENCE_SRC, "diffusionkit", "mlx")
+
 SEEDS = {"flux": 41, "sd3": 42, "vae_dec": 43, "vae_enc": 44, "sd35": 45}
 
 
 def reference_mlx_available() -> bool:
-    return os.path.exists(os.path.join(REF_MLX_DIR, "mmdit.py"))
+    return reference_shims.reference_available() and os.path.exists(os.path.join(REF_MLX_DIR, "mmdit.py"))
 
 
 def load_reference_mlx(name: str):
-    """import /root/reference/.../mlx/<name>.py as `_refmlx.<name>` without running the package's __init__ (which pulls
+    """import <reference>/python/src/diffusionkit/mlx/<name>.py as `_refmlx.<name>` without running the package's __init__ (which pulls
     in tokenizers, PIL pipelines and Hugging Face downloads)"""
     mlx_standin.install()
     reference_shims.install()            # argmaxtools.utils.get_logger
@@ -169,7 +171,7 @@ def load_reference_pipeline_package():
         tu.InferenceContextSpec = type("InferenceContextSpec", (), {})
         sys.modules["argmaxtools.test_utils"] = tu
         sys.modules["argmaxtools"].test_utils = tu
-    src = "/root/reference/python/src"
+    src = reference_shims.REFERENCE_SRC
     if src not in sys.path:
         sys.path.insert(0, src)
     return importlib.import_module("diffusionkit.mlx")
@@ -236,7 +238,7 @@ def make_inputs(kind):
 
 
 if __name__ == "__main__":
-    assert reference_mlx_available(), "needs /root/reference"
+    assert reference_mlx_available(), "set DIFFUSIONKIT_REFERENCE to an argmaxinc/DiffusionKit checkout"
     for kind in ("flux", "sd3", "sd35"):
         latent, text, pooled, timesteps, ti = make_inputs(kind)
         y = run_reference_mmdit(kind, latent, text, pooled, timesteps, ti)

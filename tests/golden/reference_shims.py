@@ -1,5 +1,5 @@
 """Stand-ins that let the reference's OWN PyTorch modules (python/src/diffusionkit/torch/mmdit.py and vae.py — real
-reference code, imported from /root/reference, never copied) run in this container.
+reference code, imported from a checkout named by $DIFFUSIONKIT_REFERENCE, never copied) run under plain PyTorch.
 
 Those two files import four generic building blocks from the un-vendored dependency `argmaxtools>=0.1.13`
 (setup.py:29), which is not installed here:
@@ -9,7 +9,7 @@ The classes below restate them from how the reference uses them and from the che
 (torch/mmdit.py:424-497: every projection is a 1x1 Conv2d over the (batch, channels, 1, sequence) layout, k_proj has no
 bias).  Everything else that executes — patch embedding, positional-embedding crop, timestep / pooled adapters, adaLN
 chunk order, pre/post-SDPA wiring, gating, final layer, unpatchify, the whole VAE decoder topology — is the reference's
-code.  Test infrastructure only (tests/golden/make_reference_golden.py, tests/test_reference_pin_cpu.py).
+code.  Test infrastructure only (tests/golden/make_reference_golden.py, make_reference_pins.py).
 """
 import enum
 import importlib.util
@@ -21,7 +21,9 @@ import types
 import torch
 import torch.nn as nn
 
-REFERENCE_TORCH_DIR = "/root/reference/python/src/diffusionkit/torch"
+# python/src of an argmaxinc/DiffusionKit checkout; only the golden-data generators under tests/golden/ read it
+REFERENCE_SRC = os.path.join(os.environ.get("DIFFUSIONKIT_REFERENCE", ""), "python", "src")
+REFERENCE_TORCH_DIR = os.path.join(REFERENCE_SRC, "diffusionkit", "torch")
 
 
 class LayerNorm(nn.Module):
@@ -111,7 +113,7 @@ def install():
 
 
 def load_reference_module(name: str):
-    """import /root/reference/python/src/diffusionkit/torch/<name>.py by path (no package __init__ side effects)"""
+    """import <reference>/python/src/diffusionkit/torch/<name>.py by path (no package __init__ side effects)"""
     install()
     path = os.path.join(REFERENCE_TORCH_DIR, name + ".py")
     spec = importlib.util.spec_from_file_location(f"_reference_torch_{name}", path)
@@ -121,4 +123,4 @@ def load_reference_module(name: str):
 
 
 def reference_available() -> bool:
-    return os.path.exists(os.path.join(REFERENCE_TORCH_DIR, "mmdit.py"))
+    return bool(os.environ.get("DIFFUSIONKIT_REFERENCE")) and os.path.exists(os.path.join(REFERENCE_TORCH_DIR, "mmdit.py"))

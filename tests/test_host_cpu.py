@@ -42,14 +42,16 @@ def test_library_loads_and_exports_every_symbol():
 
 
 def test_no_cpu_fallback():
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    with pytest.raises(dk.DkError):
-        FluxPipeline(w16=True, a16=True)
-    from diffusionkit_b200 import ops
-
-    with pytest.raises(dk.DkError):
-        ops.gemm(torch.zeros(8, 8, dtype=torch.bfloat16), torch.zeros(8, 8, dtype=torch.bfloat16))
+    """without a CUDA device the pipeline and the ops refuse with DkError; the devices are hidden from a child process,
+    so this is checked on a machine with a GPU too"""
+    code = ("import sys\nsys.path.insert(0, sys.argv[1])\nimport torch\nimport diffusionkit_b200 as dk\n"
+            "from diffusionkit_b200 import ops\nassert not torch.cuda.is_available()\n"
+            "for call in (lambda: dk.FluxPipeline(w16=True, a16=True),\n"
+            "             lambda: ops.gemm(torch.zeros(8, 8, dtype=torch.bfloat16), torch.zeros(8, 8, dtype=torch.bfloat16))):\n"
+            "    try:\n        call()\n    except dk.DkError as e:\n        print('DkError:', e)\n")
+    out = subprocess.run([sys.executable, "-c", code, ROOT], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                         capture_output=True, text=True, timeout=300)
+    assert out.returncode == 0 and out.stdout.count("DkError:") == 2, out.stdout + out.stderr
 
 
 def test_pipeline_argument_errors():
@@ -57,11 +59,16 @@ def test_pipeline_argument_errors():
         DiffusionPipeline(w16=True, a16=True, model_version="no/such-model")
     with pytest.raises(NotImplementedError):
         DiffusionPipeline(w16=False, a16=False)          # fp32 path not provided
-    from diffusionkit_b200._lib import DkError
-
-    with pytest.raises(DkError):                         # valid arguments, but no CUDA device here: refuses loudly
-        FluxPipeline(w16=True, a16=True, quantize_mmdit=True,
-                     model_version="argmaxinc/mlx-FLUX.1-schnell-4bit-quantized")
+    # valid arguments, but no CUDA device: refuses loudly.  The devices are hidden from a child process, so this is
+    # checked on a machine with a GPU too (where the same call would build the model).
+    code = ("import sys\nsys.path.insert(0, sys.argv[1])\nfrom diffusionkit_b200 import FluxPipeline\n"
+            "from diffusionkit_b200._lib import DkError\ntry:\n"
+            "    FluxPipeline(w16=True, a16=True, quantize_mmdit=True,\n"
+            "                 model_version='argmaxinc/mlx-FLUX.1-schnell-4bit-quantized')\n"
+            "except DkError as e:\n    print('DkError:', e)\n")
+    out = subprocess.run([sys.executable, "-c", code, ROOT], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                         capture_output=True, text=True, timeout=300)
+    assert out.returncode == 0 and "DkError:" in out.stdout, out.stdout + out.stderr
 
 
 def test_presets_match_reference_values():
@@ -307,6 +314,33 @@ def test_bench_vae_roofline_helper():
     assert 0.9 < r["dram_over_model"] < 1.0 and 0.15 < r["hbm_frac"] < 0.25
     r2 = bench.vae_roofline(3.4, 1, 64, peaks)                       # C2: 512^2, a quarter of the pixels
     assert abs(r2["tflop_per_image"] - 10.472 / 4) < 1e-9 and abs(r2["dram_gb_model"] - 13.46 / 4) < 1e-9
+
+
+def test_bench_dump_outputs(tmp_path):
+    """bench.py --dump-outputs: float32 .npy files under 64 MB in all; arrays over their share are sampled at the same
+    positions in every run (C4 shapes: 4 images of 1024^2)"""
+    import importlib.util
+
+    import numpy as np
+
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    g = torch.Generator().manual_seed(0)
+    images = torch.rand((4, 1024, 1024, 3), generator=g)
+    arrays = {"latents": torch.randn((4, 128, 128, 16), generator=g), "images": images,
+              "images_uint8": (images * 255).to(torch.uint8)}
+    a = bench.dump_outputs(str(tmp_path / "a"), arrays)
+    b = bench.dump_outputs(str(tmp_path / "b"), arrays)
+    assert a == b == {"latents.npy": [4, 128, 128, 16], "images_sample.npy": [a["images_sample.npy"][0]],
+                      "images_uint8_sample.npy": [a["images_sample.npy"][0]]}
+    assert sum(os.path.getsize(p) for p in (tmp_path / "a").iterdir()) < 64e6
+    for name in a:
+        x, y = np.load(tmp_path / "a" / name), np.load(tmp_path / "b" / name)
+        assert x.dtype == np.float32 and np.array_equal(x, y), name
+    assert np.array_equal(np.load(tmp_path / "a" / "latents.npy"), arrays["latents"].numpy())
+    img, u8 = np.load(tmp_path / "a" / "images_sample.npy"), np.load(tmp_path / "a" / "images_uint8_sample.npy")
+    assert np.array_equal((img * 255).astype(np.uint8).astype(np.float32), u8)     # same positions in both arrays
 
 
 def test_attention_trace_numbers_quoted_in_design():

@@ -1,6 +1,8 @@
-"""CPU: the oracle against the reference's MLX SOURCE (mlx/mmdit.py, vae.py, sampler.py), executed from /root/reference on
-tests/golden/mlx_standin.py — a torch-backed stand-in for the MLX primitives those files call.  Fixtures committed by
-tests/golden/make_reference_mlx_golden.py (fp32); re-generated live whenever /root/reference is mounted.
+"""CPU: the oracle against the reference's MLX SOURCE (mlx/mmdit.py, vae.py, sampler.py, clip.py, t5.py, tokenizer.py,
+model_io.py, __init__.py), executed from a reference checkout on tests/golden/mlx_standin.py — a torch-backed stand-in
+for the MLX primitives those files call.  Fixtures committed by tests/golden/make_reference_mlx_golden.py (fp32) and
+tests/golden/make_reference_pins.py; re-running those against a reference checkout and diffing the fixtures checks that
+the reference has not drifted.
 
 What this pins: every line of the reference above the primitive level, for BOTH model families — FLUX (dual + single-
 stream blocks, RoPE tables and rotation, QK-RMSNorm, reshape patchify / unpack, [text | image] order, shared fc2/o_proj
@@ -21,10 +23,14 @@ from oracle import sampler_ref as sr
 from oracle.mmdit_ref import MMDiTRef
 from oracle.vae_ref import VAEDecoderRef, VAEEncoderRef
 from tests.golden import make_reference_mlx_golden as mk
+from tests.golden import make_reference_pins as pins
 from tests.oracle_bridge import ref_config
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-LIVE = pytest.mark.skipif(not mk.reference_mlx_available(), reason="/root/reference is only mounted in the build container")
+
+
+def _pins():
+    return np.load(os.path.join(GOLD, "reference_pins.npz")), json.load(open(os.path.join(GOLD, "reference_pins.json")))
 
 
 def _oracle_mmdit(kind, latent, text, pooled, timesteps, ti):
@@ -79,44 +85,37 @@ def test_oracle_sampler_matches_reference_mlx_source():
         assert abs(float(ns) - w["noise_scaling_0.7"]) < 1e-6
 
 
-@LIVE
 def test_mlxsrc_fixtures_are_what_the_reference_source_produces_today():
+    """the MMDiT fixtures hold the reference's outputs for the inputs make_inputs() draws today (to the last bits, which
+    torch.randn's CPU kernels vary between instruction sets)"""
     for kind in ("flux", "sd3", "sd35"):
         latent, text, pooled, timesteps, ti = mk.make_inputs(kind)
         g = np.load(os.path.join(GOLD, f"reference_mlxsrc_{kind}_mmdit.npz"))
-        y = mk.run_reference_mmdit(kind, latent, text, pooled, timesteps, ti)
-        assert np.allclose(y.numpy(), g["out"], atol=1e-6), kind
-    assert mk.run_reference_sampler() == json.load(open(os.path.join(GOLD, "reference_mlxsrc_sampler.json")))
+        for k, v in (("latent", latent), ("text", text), ("pooled", pooled), ("timesteps", timesteps)):
+            assert np.allclose(g[k], v.numpy(), rtol=1e-5, atol=1e-5), (kind, k)
+        assert int(g["t_index"]) == ti and g["out"].shape == latent.shape, kind
+    assert set(json.load(open(os.path.join(GOLD, "reference_mlxsrc_sampler.json")))) == {"sd3_shift3", "flux_shift1",
+                                                                                        "flux_shift3"}
 
 
-@LIVE
 def test_reference_16bit_quirks_match_the_oracle_flags():
     """the reference source run with 16-bit activations on the stand-in (bf16 sinusoid, Q5; per-op rounding) stays within
     16-bit tolerance of the oracle's act_dtype emulation — a looser check that the dtype plumbing is the same"""
-    import sys
     from dataclasses import replace
 
-    mx = sys.modules["mlx.core"]
-    rcfg_mod, rmm = mk.load_reference_mlx("config"), mk.load_reference_mlx("mmdit")
+    g, _ = _pins()
+    out = torch.from_numpy(g["mlx_16bit_flux_mmdit"])
     flux, _ = mk.pin_configs()
     cfg16 = replace(flux, dtype=torch.bfloat16, float16_dtype=torch.bfloat16)
     params = init_params(mmdit_param_specs(cfg16), seed=mk.SEEDS["flux"], dtype=torch.float32)
     p16 = {k: v.to(torch.bfloat16) for k, v in params.items()}
-    rc = mk.reference_config(rcfg_mod, cfg16)
-    rc.dtype = rc.float16_dtype = mx.bfloat16
-    model = rmm.MMDiT(rc)
-    model.load_weights([(k, mx.array(v.clone())) for k, v in p16.items()], strict=True)
     latent, text, pooled, timesteps, ti = mk.make_inputs("flux")
     l16, t16, pl16 = [x.to(torch.bfloat16) for x in (latent, text, pooled)]
-    ts16 = timesteps.to(torch.bfloat16)
-    model.cache_modulation_params(mx.array(pl16.clone()), mx.array(ts16.clone()))
-    out = model(latent_image_embeddings=mx.array(l16.clone()),
-                token_level_text_embeddings=mx.array(t16.clone()[:, :, None, :]),
-                timestep=mx.repeat(mx.array(ts16.clone())[ti][None], 2, axis=0)).t.float()
     ref = MMDiTRef(ref_config(cfg16), {k: v.float() for k, v in p16.items()}, act_dtype=torch.bfloat16)
-    tsf = ts16.float()
+    tsf = timesteps.to(torch.bfloat16).float()
     ref.cache_modulation_params(pl16.float(), tsf)
     got = ref(l16.float(), t16.float(), tsf[ti].repeat(2))
+    assert got.shape == out.shape
     rel = float((got - out).norm() / out.norm())
     assert rel < 2e-2, rel
 
@@ -153,300 +152,134 @@ def test_oracle_denoise_loop_matches_reference_pipeline_source(kind):
     assert torch.allclose(img, torch.from_numpy(g["image"]), atol=5e-4), float((img - torch.from_numpy(g["image"])).abs().max())
 
 
-@LIVE
 def test_pipeline_fixtures_are_what_the_reference_source_produces_today():
+    """the pipeline fixtures hold the reference's outputs for the inputs make_pipeline_inputs() draws today, and
+    the reference loop ran one iteration per step"""
+    _, meta = _pins()
     for kind, (steps, cfgw, shift, lat, seed, _) in mk.PIPELINE_CASES.items():
         cond, pooled = mk.make_pipeline_inputs(kind)
-        latent, image, sig, n_iter = mk.run_reference_pipeline(kind, cond, pooled, steps, cfgw, shift, lat, seed)
         g = np.load(os.path.join(GOLD, f"reference_mlxsrc_{kind}_pipeline.npz"))
-        assert n_iter == steps
-        assert np.allclose(latent.numpy(), g["latent"], atol=1e-5), kind
+        assert np.allclose(g["cond"], cond.numpy(), rtol=1e-5, atol=1e-5), kind
+        assert np.allclose(g["pooled"], pooled.numpy(), rtol=1e-5, atol=1e-5), kind
+        assert meta["pipeline_iterations"][kind] == steps
+        assert g["latent"].shape == (1, lat[0], lat[1], 16), kind
 
 
-@LIVE
 def test_text_encoder_oracles_match_reference_mlx_source():
     """CLIPTextModel (mlx/clip.py) and SD3T5Encoder (mlx/t5.py) of the reference, run on the stand-in, vs oracle/text_ref.py
     (which tests/test_text_cpu.py separately pins against transformers)"""
-    import sys
-
-    from transformers import T5Config
-
-    from diffusionkit_b200.config import tiny_clip_config, tiny_t5_config
-    from diffusionkit_b200.text_encoders import clip_param_specs, t5_param_specs
     from oracle.text_ref import CLIPTextModelRef, T5EncoderRef
 
-    dm = mk.load_reference_pipeline_package()
-    mx = sys.modules["mlx.core"]
-    from diffusionkit.mlx import clip as rclip, config as rcfg, t5 as rt5
-
-    for act, proj in (("quick_gelu", True), ("gelu", False)):
-        cfg = tiny_clip_config(projection=proj, act=act)
-        params = init_params(clip_param_specs(cfg), seed=71, dtype=torch.float32)
-        model = rclip.CLIPTextModel(rcfg.CLIPTextModelConfig(
-            num_layers=cfg.num_layers, model_dims=cfg.model_dims, num_heads=cfg.num_heads, max_length=cfg.max_length,
-            vocab_size=cfg.vocab_size, projection_dim=cfg.projection_dim, hidden_act=cfg.hidden_act))
-        model.load_weights(mk.to_mx(params), strict=True)
-        tokens = torch.randint(1, cfg.vocab_size - 1, (2, 24), generator=torch.Generator().manual_seed(5))
-        tokens[0, 9] = tokens[1, 23] = cfg.vocab_size - 1
-        out = model(mx.array(tokens.to(torch.int32)))
-        pooled, last, hidden = CLIPTextModelRef(params, cfg.num_layers, cfg.num_heads, act)(tokens)
-        assert torch.allclose(last, out.last_hidden_state.t, atol=3e-4, rtol=1e-4)
-        assert torch.allclose(pooled, out.pooled_output.t, atol=3e-4, rtol=1e-4)
-        assert torch.allclose(hidden[-2], out.hidden_states[-2].t, atol=3e-4, rtol=1e-4)
-
-    tc = tiny_t5_config()
-    tparams = init_params(t5_param_specs(tc), seed=72, dtype=torch.float32)
-    tparams["encoder.relative_attention_bias.embeddings.weight"] *= 30.0
-    tparams["wte.weight"] *= 30.0
-    hf_cfg = T5Config(vocab_size=tc.vocab_size, d_model=tc.d_model, d_kv=tc.d_kv, d_ff=tc.d_ff, num_layers=tc.num_layers,
-                      num_heads=tc.num_heads, feed_forward_proj="gated-gelu", relative_attention_num_buckets=32,
-                      relative_attention_max_distance=128, layer_norm_epsilon=1e-6)
-    enc = rt5.SD3T5Encoder(hf_cfg, low_memory_mode=False)
-    enc.load_weights(mk.to_mx(tparams), strict=True)
-    tokens = torch.randint(0, tc.vocab_size, (2, 160), generator=torch.Generator().manual_seed(6))
-    want = enc(mx.array(tokens.to(torch.int32))).t
-    got = T5EncoderRef(tparams, tc.num_layers, tc.num_heads)(tokens)
-    assert torch.allclose(got, want, atol=5e-4, rtol=1e-4), float((got - want).abs().max())
+    g, _ = _pins()
+    clip, (tc, tparams, ttokens) = pins.text_encoder_cases()
+    for name, cfg, params, tokens in clip:
+        pooled, last, hidden = CLIPTextModelRef(params, cfg.num_layers, cfg.num_heads, cfg.hidden_act)(tokens)
+        for got, key in ((last, "last"), (pooled, "pooled"), (hidden[-2], "hidden_m2")):
+            pins.assert_close(g, f"{name}_{key}", got, atol=3e-4, rtol=1e-4)
+    pins.assert_close(g, "t5_out", T5EncoderRef(tparams, tc.num_layers, tc.num_heads)(ttokens), atol=5e-4, rtol=1e-4)
 
 
-@LIVE
 def test_checkpoint_key_maps_match_reference_mlx_loaders():
     """SURVEY.md §8 row f1 against the reference's own MLX loader functions (mlx/model_io.py:130-636), run on the stand-in:
-    an upstream-layout checkpoint (BFL FLUX, Stability SD3, LDM VAE, HF T5 / CLIP) goes through the reference's
-    *_state_dict_adjustments and through diffusionkit_b200.model_io; both must give the same names and tensors, and the
-    reference's result must load into the reference module tree with strict=True"""
-    import sys
-
+    an upstream-layout checkpoint (BFL FLUX, Stability SD3, LDM VAE, HF T5) goes through the reference's
+    *_state_dict_adjustments (for FLUX: what Module.update leaves in the reference module tree) and through
+    diffusionkit_b200.model_io; both must give the same names and bit-identical tensors"""
     from diffusionkit_b200 import model_io
-    from diffusionkit_b200.config import VAEDecoderConfig, VAEEncoderConfig, tiny_t5_config
-    from diffusionkit_b200.text_encoders import t5_param_specs
-    from tests.test_model_io_cpu import _flux_upstream, _sd3_upstream, _vae_upstream
 
-    dm = mk.load_reference_pipeline_package()
-    mx = sys.modules["mlx.core"]
-    rio = dm.model_io
-    flux, sd3 = mk.pin_configs()
-
-    def as_mx(d):
-        return {k: mx.array(v.clone()) for k, v in d.items()}
-
-    def same(ref_dict, mine, allow_missing=()):
-        ref_t = {k: v.t for k, v in ref_dict.items()}
-        assert set(ref_t) - set(allow_missing) == set(mine), (sorted(set(ref_t) ^ set(mine))[:6])
-        for k, v in mine.items():
-            assert ref_t[k].shape == v.shape and torch.equal(ref_t[k], v), k
-
-    # FLUX (BFL layout): qkv / linear1 / linear2 splits, shared bias, scale -> weight renames
-    fparams = init_params(mmdit_param_specs(flux), seed=81, dtype=torch.float32)
-    fup = _flux_upstream(fparams, flux)
-    ref_flux = rio.flux_state_dict_adjustments(as_mx(fup), prefix="", hidden_size=flux.hidden_size,
-                                               mlp_ratio=flux.mlp_ratio)
-    # the reference loads FLUX with Module.update (model_io.py:776), which ignores keys its module tree does not have
-    # (k_proj.bias: quirk Q3; guidance_in.*: quirk Q1) — compare what actually ends up in the model
-    from diffusionkit.mlx import config as rcfg_mod, mmdit as rmm
-    from mlx.utils import tree_flatten, tree_unflatten
-
-    model = rmm.MMDiT(mk.reference_config(rcfg_mod, flux))
-    untouched = {k for k, _ in tree_flatten(model.parameters())}
-    model.update(tree_unflatten(list(ref_flux.items())))
-    effective = dict(tree_flatten(model.parameters()))
-    assert set(effective) == untouched                       # update added nothing
-    assert any(k.endswith("k_proj.bias") for k in ref_flux) and not any(k.endswith("k_proj.bias") for k in effective)
-    same(effective, model_io.flux_checkpoint_to_params(fup, flux.hidden_size, flux.mlp_ratio))
-
-    # SD3 (Stability layout, same file also holds VAE tensors)
-    sparams = init_params(mmdit_param_specs(sd3), seed=82, dtype=torch.float32)
-    sup = _sd3_upstream(sparams, sd3)
-    ref_sd3 = rio.mmdit_state_dict_adjustments(as_mx(sup), prefix="model.diffusion_model.")
-    same(ref_sd3, model_io.sd3_checkpoint_to_params(sup))
-
-    # VAE decoder / encoder (LDM layout behind first_stage_model.)
-    from diffusionkit_b200.weights import vae_encoder_param_specs as enc_specs
-
-    dparams = init_params(vae_decoder_param_specs(VAEDecoderConfig()), seed=83, dtype=torch.float32)
-    dup = _vae_upstream(dparams, prefix="first_stage_model.decoder.")
-    same(rio.vae_decoder_state_dict_adjustments(as_mx(dup), prefix="first_stage_model.decoder."),
-         model_io.vae_decoder_checkpoint_to_params(dup))
-    eparams = init_params(enc_specs(VAEEncoderConfig()), seed=84, dtype=torch.float32)
-    eup = _vae_upstream(eparams, prefix="first_stage_model.encoder.")
-    same(rio.vae_encoder_state_dict_adjustments(as_mx(eup), prefix="first_stage_model.encoder."),
-         model_io.vae_encoder_checkpoint_to_params(eup))
-
-    # T5 (HF T5EncoderModel names)
-    tc = tiny_t5_config()
-    tparams = init_params(t5_param_specs(tc), seed=85, dtype=torch.float32)
-    hf = {}
-    for k, v in tparams.items():
-        if k == "wte.weight":
-            hf["encoder.embed_tokens.weight"] = v
-            hf["shared.weight"] = v
-        elif k == "encoder.ln.weight":
-            hf["encoder.final_layer_norm.weight"] = v
-        elif k == "encoder.relative_attention_bias.embeddings.weight":
-            hf["encoder.block.0.layer.0.SelfAttention.relative_attention_bias.weight"] = v
-        else:
-            i, rest = k.split(".")[2], ".".join(k.split(".")[3:])
-            rest = (rest.replace("attention.query_proj", "layer.0.SelfAttention.q")
-                    .replace("attention.key_proj", "layer.0.SelfAttention.k")
-                    .replace("attention.value_proj", "layer.0.SelfAttention.v")
-                    .replace("attention.out_proj", "layer.0.SelfAttention.o").replace("ln1", "layer.0.layer_norm")
-                    .replace("ln2", "layer.1.layer_norm").replace("dense.", "layer.1.DenseReluDense."))
-            hf[f"encoder.block.{i}.{rest}"] = v
-    same(rio.t5_encoder_state_dict_adjustments(as_mx(hf), prefix=""), model_io.t5_checkpoint_to_params(hf))
+    _, meta = _pins()
+    flux, _ = mk.pin_configs()
+    ck = pins.key_map_checkpoints()
+    mine = {"flux": model_io.flux_checkpoint_to_params(ck["flux"], flux.hidden_size, flux.mlp_ratio),
+            "sd3": model_io.sd3_checkpoint_to_params(ck["sd3"]),
+            "vae_decoder": model_io.vae_decoder_checkpoint_to_params(ck["vae_decoder"]),
+            "vae_encoder": model_io.vae_encoder_checkpoint_to_params(ck["vae_encoder"]),
+            "t5": model_io.t5_checkpoint_to_params(ck["t5"])}
+    assert set(mine) == set(meta["key_maps"])
+    for part, params in mine.items():
+        want = meta["key_maps"][part]
+        assert set(want) == set(params), (part, sorted(set(want) ^ set(params))[:6])
+        for k, v in params.items():
+            assert pins.digest(v) == want[k], (part, k)
 
 
-@LIVE
 def test_clip_tokenizer_matches_reference_tokenizer(tmp_path):
     """diffusionkit_b200.tokenizer.Tokenizer vs the reference's own class (mlx/tokenizer.py:14-122) on the synthetic
     vocabulary (tests/test_text_cpu.py also checks it against transformers' CLIPTokenizer)"""
     from diffusionkit_b200.tokenizer import load_tokenizer
     from tests.test_text_cpu import _synthetic_clip_vocab
 
-    mk.load_reference_pipeline_package()
-    from diffusionkit.mlx import tokenizer as rtok
-
+    want = _pins()[1]["tokenizer"]
     vf, mf, vocab = _synthetic_clip_vocab(tmp_path)
     mine = load_tokenizer(vf, mf, pad_with_eos=True)
-    ref = rtok.Tokenizer(mine.bpe_ranks, mine.vocab, pad_with_eos=True)
-    for text in ["a photo of a cat", "The  astronaut riding a horse on Mars!!", "cats, cats , 42 cats!", "a",
-                 " ".join(["cat"] * 200)]:
-        assert mine.tokenize(text) == ref.tokenize(text), text
-    assert mine.eos_token == ref.eos_token and mine.bos_token == ref.bos_token
+    assert len(want["tokens"]) == len(pins.TOKENIZER_TEXTS)
+    for text, ref_tokens in zip(pins.TOKENIZER_TEXTS, want["tokens"]):
+        assert [int(t) for t in mine.tokenize(text)] == ref_tokens, text
+    assert mine.eos_token == want["eos_token"] and mine.bos_token == want["bos_token"]
 
 
-class _WordTokenizer:
-    """minimal object with the interface the pipelines' _tokenize uses (tokenize / max_length / pad flags / eos_token)"""
-
-    def __init__(self, max_length, pad_with_eos, eos=99, bos=None, vocab_size=100):
-        self.max_length, self.pad_with_eos, self.pad_to_max_length = max_length, pad_with_eos, True
-        self.eos_token, self._bos, self._v = eos, bos, vocab_size
-
-    def tokenize(self, text):
-        ids = [1 + (sum(map(ord, w)) % (self._v - 3)) for w in text.split()][: self.max_length - 2]
-        return ([self._bos] if self._bos is not None else []) + ids + [self.eos_token]
-
-
-@LIVE
 def test_encode_text_composition_matches_reference_pipeline_source():
     """the reference's own _tokenize / encode_text of both pipelines (mlx/__init__.py:174-251, 642-671) on the stand-in, vs
     the product's host-side _tokenize and the oracle's encode_text_* composition"""
-    import sys
-
-    from transformers import T5Config
-
-    from diffusionkit_b200.config import CLIPTextModelConfig, T5EncoderConfig
     from diffusionkit_b200.pipeline import DiffusionPipeline as OurPipe
-    from diffusionkit_b200.text_encoders import clip_param_specs, t5_param_specs
     from oracle.text_ref import CLIPTextModelRef, T5EncoderRef, encode_text_flux, encode_text_sd3, tokenize_pair
 
-    dm = mk.load_reference_pipeline_package()
-    mx = sys.modules["mlx.core"]
-    from diffusionkit.mlx import clip as rclip, config as rcfg, t5 as rt5
-
-    cl = CLIPTextModelConfig(num_layers=2, model_dims=128, num_heads=2, vocab_size=100, projection_dim=None)
-    cg = CLIPTextModelConfig(num_layers=2, model_dims=192, num_heads=3, vocab_size=100, projection_dim=192, hidden_act="gelu")
-    tc = T5EncoderConfig(vocab_size=100, d_model=4096, d_kv=64, d_ff=128, num_layers=1, num_heads=2)
-    pl = init_params(clip_param_specs(cl), seed=91, dtype=torch.float32)
-    pg = init_params(clip_param_specs(cg), seed=92, dtype=torch.float32)
-    pt = init_params(t5_param_specs(tc), seed=93, dtype=torch.float32)
-    pt["wte.weight"] *= 30.0
-
-    def ref_clip(c, p):
-        m = rclip.CLIPTextModel(rcfg.CLIPTextModelConfig(num_layers=c.num_layers, model_dims=c.model_dims,
-                                                         num_heads=c.num_heads, max_length=c.max_length,
-                                                         vocab_size=c.vocab_size, projection_dim=c.projection_dim,
-                                                         hidden_act=c.hidden_act))
-        m.load_weights(mk.to_mx(p), strict=True)
-        return m
-
-    t5 = rt5.SD3T5Encoder(T5Config(vocab_size=tc.vocab_size, d_model=tc.d_model, d_kv=tc.d_kv, d_ff=tc.d_ff,
-                                   num_layers=tc.num_layers, num_heads=tc.num_heads, feed_forward_proj="gated-gelu",
-                                   relative_attention_num_buckets=32, relative_attention_max_distance=128,
-                                   layer_norm_epsilon=1e-6), low_memory_mode=False)
-    t5.load_weights(mk.to_mx(pt), strict=True)
-    tok_l, tok_g = _WordTokenizer(77, True, bos=98), _WordTokenizer(77, False, bos=98)
-    text, neg = "a photo of an astronaut riding a horse on mars", "blurry low quality"
-    o_l = CLIPTextModelRef(pl, cl.num_layers, cl.num_heads, cl.hidden_act)
-    o_g = CLIPTextModelRef(pg, cg.num_layers, cg.num_heads, cg.hidden_act)
-    o_t = T5EncoderRef(pt, tc.num_layers, tc.num_heads)
+    g, meta = _pins()
+    s = pins.encode_text_setup()
+    cl, cg, tc = s["cl"], s["cg"], s["tc"]
+    o_l = CLIPTextModelRef(s["pl"], cl.num_layers, cl.num_heads, cl.hidden_act)
+    o_g = CLIPTextModelRef(s["pg"], cg.num_layers, cg.num_heads, cg.hidden_act)
+    o_t = T5EncoderRef(s["pt"], tc.num_layers, tc.num_heads)
+    tok_l, tok_g, text, neg = s["tok_l"], s["tok_g"], s["text"], s["neg"]
 
     for kind in ("sd3", "flux"):
-        Pipe = dm.DiffusionPipeline if kind == "sd3" else dm.FluxPipeline
-        pipe = object.__new__(Pipe)
-        pipe.clip_l, pipe.clip_g, pipe.t5_encoder = ref_clip(cl, pl), ref_clip(cg, pg), t5
-        pipe.tokenizer_l, pipe.tokenizer_g = tok_l, tok_g
-        t5_len = 64 if kind == "sd3" else 48
-        pipe.t5_tokenizer = _WordTokenizer(t5_len, False, eos=1)
-        pipe.use_t5 = True
-        pipe.model_version = "pin"
-        dm.T5_MAX_LENGTH["pin"] = t5_len
+        t5_len = s["t5_len"][kind]
+        tok_t5 = pins.WordTokenizer(t5_len, False, eos=1)
         for cfgw in (5.0, 0.0):
+            case = f"{kind}_cfg{int(cfgw)}"
             # token batching: reference _tokenize == product _tokenize == oracle tokenize_pair
             n = neg if cfgw > 1 else None
-            for tk in (tok_l, tok_g, pipe.t5_tokenizer):
-                want_tok = torch.tensor(pipe._tokenize(tk, text, n).tolist())
-                assert torch.equal(OurPipe._tokenize(None, tk, text, n), want_tok)
-                assert torch.equal(tokenize_pair(tk, text, n), want_tok)
-            cond, pooled = pipe.encode_text(text, cfgw, neg)
-            tl, tg, tt = [tokenize_pair(tk, text, n) for tk in (tok_l, tok_g, pipe.t5_tokenizer)]
+            for tk, want in zip((tok_l, tok_g, tok_t5), meta["encode_text_tokens"][case]):
+                want_tok = torch.tensor(want)
+                assert torch.equal(OurPipe._tokenize(None, tk, text, n), want_tok), case
+                assert torch.equal(tokenize_pair(tk, text, n), want_tok), case
+            tl, tg, tt = [tokenize_pair(tk, text, n) for tk in (tok_l, tok_g, tok_t5)]
             if kind == "sd3":
                 got_c, got_p = encode_text_sd3(o_l, o_g, o_t, tl, tg, tt)
-                assert cond.shape == (2, 77 + t5_len, 4096) and pooled.shape == (2, 128 + 192)
+                assert got_c.shape == (2, 77 + t5_len, 4096) and got_p.shape == (2, 128 + 192)
             else:
                 got_c, got_p = encode_text_flux(o_l, o_t, tl, tt, t5_len)
-                assert cond.shape == (1, t5_len, 4096) and pooled.shape == (1, 128)
-            assert torch.allclose(got_c, cond.t, atol=5e-4, rtol=1e-4), (kind, cfgw)
-            assert torch.allclose(got_p, pooled.t, atol=5e-4, rtol=1e-4), (kind, cfgw)
+                assert got_c.shape == (1, t5_len, 4096) and got_p.shape == (1, 128)
+            pins.assert_close(g, f"encode_text_{case}_cond", got_c, atol=5e-4, rtol=1e-4)
+            pins.assert_close(g, f"encode_text_{case}_pooled", got_p, atol=5e-4, rtol=1e-4)
 
 
-@LIVE
 def test_img2img_flow_matches_reference_pipeline_source(tmp_path):
     """image_path / denoise arguments (mlx/__init__.py:270-285, 536-551, 586-594): read_image incl. the LANCZOS resize to
     multiples of 64, VAE encoder, clipped-logvar posterior sample drawn with the SAME seeded noise as the diffusion
     noise, process_in, schedule trimming, noise_scaling with a tensor x_T — reference source on the stand-in vs the
     oracle composition the GPU check (tests/model_checks.py::check_pipeline_img2img) compares the product against"""
-    import sys
-
     from PIL import Image
 
     from diffusionkit_b200.config import VAEEncoderConfig
     from diffusionkit_b200.pipeline import DiffusionPipeline as OurPipe
     from oracle.vae_ref import encode_image_to_latents, read_image_array
 
-    dm = mk.load_reference_pipeline_package()
-    mx = sys.modules["mlx.core"]
-    from diffusionkit.mlx import config as rcfg_mod, mmdit as rmm, vae as rvae
-
+    g, meta = _pins()
+    steps, denoise, seed = pins.IMG2IMG["steps"], pins.IMG2IMG["denoise"], pins.IMG2IMG["seed"]
+    latent = torch.from_numpy(g["img2img_latent"])
+    assert meta["img2img_iterations"] == steps - int(steps * (1 - denoise)) and latent.shape == (1, 8, 16, 16)
     flux, _ = mk.pin_configs()
     params = init_params(mmdit_param_specs(flux), seed=mk.SEEDS["flux"], dtype=torch.float32)
     ecfg = VAEEncoderConfig(block_out_channels=(32, 64, 64, 64), layers_per_block=2)
     eparams = init_params(vae_encoder_param_specs(ecfg), seed=mk.SEEDS["vae_enc"], dtype=torch.float32)
-    pipe = object.__new__(dm.FluxPipeline)
-    pipe.mmdit = rmm.MMDiT(mk.reference_config(rcfg_mod, flux))
-    pipe.mmdit.load_weights(mk.to_mx(params), strict=True)
-    pipe.encoder = rvae.VAEEncoder(in_channels=3, out_channels=32, block_out_channels=list(ecfg.block_out_channels),
-                                   layers_per_block=ecfg.layers_per_block, resnet_groups=32)
-    pipe.encoder.load_weights(mk.to_mx(eparams), strict=True)
-    pipe.sampler, pipe.latent_format = dm.FluxSampler(shift=1.0), dm.FluxLatentFormat()
-    pipe.activation_dtype = pipe.dtype = pipe.float16_dtype = mx.float32
-    pipe.load_mmdit = lambda only_modulation_dict=False: [(k, mx.array(v.clone())) for k, v in params.items()
-                                                          if "adaLN" in k]
-    rng = np.random.RandomState(3)
-    img = (rng.rand(100, 150, 3) * 255).astype(np.uint8)            # not a multiple of 64: resized to 64 x 128
     path = str(tmp_path / "in.png")
-    Image.fromarray(img).save(path)
+    Image.fromarray(pins.img2img_image()).save(path)
     cond, pooled = mk.make_pipeline_inputs("flux")
-    steps, denoise, seed = 4, 0.5, 9
-    latent, iter_time = pipe.denoise_latents(mx.array(cond.clone()), mx.array(pooled.clone()), num_steps=steps,
-                                             cfg_weight=0.0, latent_size=(2, 2), seed=seed, image_path=path,
-                                             denoise=denoise)
-    assert len(iter_time) == steps - int(steps * (1 - denoise)) and latent.shape == (1, 8, 16, 16)
 
     # product host side: the same pixels after the resize rule
     ours_u8 = OurPipe._load_image_u8(None, path)
-    ref_img = pipe.read_image(path).t
     assert ours_u8.shape == (64, 128, 3)
-    assert torch.allclose(read_image_array(torch.from_numpy(ours_u8)), ref_img, atol=1e-6)
+    pins.assert_close(g, "img2img_read_image", read_image_array(torch.from_numpy(ours_u8)), atol=1e-6, rtol=0)
 
     # oracle composition
     enc = VAEEncoderRef(eparams, None, ecfg.block_out_channels, ecfg.layers_per_block)
@@ -459,7 +292,7 @@ def test_img2img_flow_matches_reference_pipeline_source(tmp_path):
     x = sr.sample_euler(lambda xin, c, t: ref(xin, c, t), ref.cache_modulation_params,
                         sampler.noise_scaling(float(sig[0]), noise, x_T), sig, cond, pooled, 0.0, torch.float32)
     got = sr.process_out(x, "flux")
-    assert torch.allclose(got, latent.t, atol=2e-3, rtol=1e-3), float((got - latent.t).abs().max())
+    assert torch.allclose(got, latent, atol=2e-3, rtol=1e-3), float((got - latent).abs().max())
 
 
 def test_oracle_fullwidth_vae_matches_reference_mlx_source():
@@ -481,41 +314,24 @@ def test_oracle_fullwidth_vae_matches_reference_mlx_source():
     assert torch.allclose(e, torch.from_numpy(g["encoded"]), atol=5e-4, rtol=1e-4)
 
 
-@LIVE
 @pytest.mark.parametrize("kind", ["flux", "sd3"])
 def test_16bit_denoise_loop_emulation_tracks_reference_source(kind):
-    """The GPU tests compare the product with the oracle run in 16-bit EMULATION (act_dtype).  Here the reference's own
-    pipeline source runs with real 16-bit arrays on the stand-in (bf16 FLUX / fp16 SD3: timestep rounding and the
-    config.dtype sinusoid of quirk Q5, the rounding residue of quirk Q6, per-op rounding) and the oracle's emulation has to
-    land on the same final latent.  Measured: 5.3e-3 (FLUX) / 2.0e-3 (SD3) rel-L2 — while the reference's 16-bit run is
-    1.1e-1 / 2.7e-2 away from its own fp32 run, i.e. the emulation reproduces the reference's 16-bit behaviour, not just
-    the fp32 math."""
-    import sys
+    """The GPU tests compare the product with the oracle run in 16-bit EMULATION (act_dtype).  The reference's own
+    pipeline source ran with real 16-bit arrays on the stand-in (bf16 FLUX / fp16 SD3: timestep rounding and the
+    config.dtype sinusoid of quirk Q5, the rounding residue of quirk Q6, per-op rounding; stored by
+    tests/golden/make_reference_pins.py) and the oracle's emulation has to land on the same final latent.  Measured:
+    5.3e-3 (FLUX) / 2.0e-3 (SD3) rel-L2 — while the reference's 16-bit run is 1.1e-1 / 2.7e-2 away from its own fp32 run,
+    i.e. the emulation reproduces the reference's 16-bit behaviour, not just the fp32 math."""
     from dataclasses import replace
 
+    g, _ = _pins()
+    want = torch.from_numpy(g[f"mlx_16bit_{kind}_pipeline_latent"])
     dt = torch.bfloat16 if kind == "flux" else torch.float16
-    dm = mk.load_reference_pipeline_package()
-    mx = sys.modules["mlx.core"]
-    mdt = mx.bfloat16 if kind == "flux" else mx.float16
-    from diffusionkit.mlx import config as rcfg_mod, mmdit as rmm
-
     steps, cfgw, shift, lat, seed, _ = mk.PIPELINE_CASES[kind]
     cfg = replace(mk.pin_config(kind), dtype=dt, float16_dtype=dt)
     p16 = {k: v.to(dt) for k, v in init_params(mmdit_param_specs(cfg), seed=mk.SEEDS[kind], dtype=torch.float32).items()}
-    rc = mk.reference_config(rcfg_mod, cfg)
-    rc.dtype = rc.float16_dtype = mdt
-    pipe = object.__new__(dm.FluxPipeline if kind == "flux" else dm.DiffusionPipeline)
-    pipe.mmdit = rmm.MMDiT(rc)
-    pipe.mmdit.load_weights([(k, mx.array(v.clone())) for k, v in p16.items()], strict=True)
-    pipe.sampler = (dm.FluxSampler if kind == "flux" else dm.ModelSamplingDiscreteFlow)(shift=shift)
-    pipe.latent_format = (dm.FluxLatentFormat if kind == "flux" else dm.SD3LatentFormat)()
-    pipe.activation_dtype = pipe.dtype = pipe.float16_dtype = mdt
-    pipe.load_mmdit = lambda only_modulation_dict=False: [(k, mx.array(v.clone())) for k, v in p16.items() if "adaLN" in k]
     cond, pooled = mk.make_pipeline_inputs(kind)
     c16, pl16 = cond.to(dt), pooled.to(dt)
-    latent, _ = pipe.denoise_latents(mx.array(c16.clone()), mx.array(pl16.clone()), num_steps=steps, cfg_weight=cfgw,
-                                     latent_size=lat, seed=seed)
-    want = latent.t.float()
     sampler = sr.FluxSamplerRef(shift) if kind == "flux" else sr.ModelSamplingDiscreteFlowRef(shift)
     sig = sr.get_sigmas(sampler, steps)
     ref = MMDiTRef(ref_config(cfg), {k: v.float() for k, v in p16.items()}, act_dtype=dt)
@@ -523,5 +339,6 @@ def test_16bit_denoise_loop_emulation_tracks_reference_source(kind):
     x = sr.sample_euler(lambda xin, c, t: ref(xin, c, t), ref.cache_modulation_params, x0, sig, c16.float(), pl16.float(),
                         cfgw, dt)
     got = sr.process_out(x, "flux" if kind == "flux" else "sd3")
+    assert got.shape == want.shape
     rel = float((got - want).norm() / want.norm())
     assert rel < 2e-2, rel
