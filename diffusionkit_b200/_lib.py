@@ -87,6 +87,8 @@ SIGNATURES = {
     "dk_upsample_nearest2x": (i32, [vp, i32, vp, vp, i32, i32, i32, i32, vp]),
     "dk_softmax_rows": (i32, [vp, i32, vp, i64, i32, i64, f32, vp]),
     "dk_image_post": (i32, [vp, i32, vp, i32, vp, vp, i64, vp]),
+    "dk_inpaint_blend": (i32, [vp, vp, vp, vp, vp, i64, i32, f32, vp]),
+    "dk_image_post_masked": (i32, [vp, i32, vp, i32, vp, vp, vp, i64, vp]),
     "dk_comm_unique_id": (i32, [vp]),
     "dk_comm_init": (i32, [vp, i32, i32, vp]),
     "dk_comm_broadcast": (i32, [vp, vp, C.c_size_t, i32, vp]),

@@ -686,7 +686,18 @@ softmax_rows_kernel(T* __restrict__ x, int n, long long ld, float scale) {
   }
 }
 
-// decode tail: clip(x/2 + 0.5, 0, 1) in the activation dtype (mlx/__init__.py:583), uint8 = trunc(x * 255) (:526)
+// decode tail of one channel value: clip(x/2 + 0.5, 0, 1) in the activation dtype (mlx/__init__.py:583) and
+// uint8 = trunc(v * 255) (:526).  image_post and image_post_masked both go through these two helpers, so the
+// regenerated pixels of an inpainting composite are bit-identical to the plain decode's.
+template <typename T>
+__device__ __forceinline__ float image_post_unit(T x) {
+  const float v = round16<T>(round16<T>(Half16<T>::to_f(x) * 0.5f) + 0.5f);
+  return fminf(fmaxf(v, 0.f), 1.f);
+}
+template <typename T>
+__device__ __forceinline__ uint8_t image_post_u8(float v) {
+  return static_cast<uint8_t>(round16<T>(v * 255.f));
+}
 template <typename T>
 __global__ void image_post_kernel(const T* __restrict__ x, int c_stride, float* __restrict__ img_f32,
                                   uint8_t* __restrict__ img_u8, long long pixels) {
@@ -694,11 +705,45 @@ __global__ void image_post_kernel(const T* __restrict__ x, int c_stride, float* 
        i += static_cast<long long>(gridDim.x) * blockDim.x) {
     const long long p = i / 3;
     const int c = static_cast<int>(i % 3);
-    float v = Half16<T>::to_f(x[p * c_stride + c]);
-    v = round16<T>(round16<T>(v * 0.5f) + 0.5f);
-    v = fminf(fmaxf(v, 0.f), 1.f);
+    const float v = image_post_unit<T>(x[p * c_stride + c]);
     if (img_f32 != nullptr) img_f32[i] = v;
-    if (img_u8 != nullptr) img_u8[i] = static_cast<uint8_t>(round16<T>(v * 255.f));
+    if (img_u8 != nullptr) img_u8[i] = image_post_u8<T>(v);
+  }
+}
+// inpainting composite: img_u8 = mask ? image_post's uint8 : orig  (orig [pixels, 3] uint8, mask one byte / pixel)
+template <typename T>
+__global__ void image_post_masked_kernel(const T* __restrict__ x, int c_stride, const uint8_t* __restrict__ orig,
+                                         const uint8_t* __restrict__ mask, uint8_t* __restrict__ img_u8,
+                                         long long pixels) {
+  for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < pixels * 3;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const long long p = i / 3;
+    const int c = static_cast<int>(i % 3);
+    img_u8[i] = mask[p] ? image_post_u8<T>(image_post_unit<T>(x[p * c_stride + c])) : orig[i];
+  }
+}
+
+// inpainting re-noise of the kept latent cells after an Euler step (fp32, one float4 per thread, Q = C / 4 float4s per
+// pixel; QC > 0 fixes Q at compile time so the pixel index is a shift):
+//   x = mask ? x : sigma_next * noise + (1 - sigma_next) * x0
+// Cells being regenerated (mask != 0) read nothing but their mask byte and are not written.
+template <int QC>
+__global__ void inpaint_blend_kernel(const float4* __restrict__ x0, const float4* __restrict__ noise,
+                                     const uint8_t* __restrict__ mask, float4* __restrict__ x, long long pixels, int Q,
+                                     float sigma_next) {
+  const int q = QC > 0 ? QC : Q;
+  const long long n = pixels * q;
+  const float keep = 1.f - sigma_next;
+  for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < n;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    if (mask[i / q]) continue;
+    const float4 a = x0[i], b = noise[i];
+    float4 o;
+    o.x = sigma_next * b.x + keep * a.x;
+    o.y = sigma_next * b.y + keep * a.y;
+    o.z = sigma_next * b.z + keep * a.z;
+    o.w = sigma_next * b.w + keep * a.w;
+    x[i] = o;
   }
 }
 
@@ -1065,6 +1110,43 @@ extern "C" int dk_image_post(dk_ctx* ctx, int dtype, const void* x, int c_stride
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DK_DISPATCH(dtype, (image_post_kernel<T><<<grid_for(pixels * 3, 256, ctx->sm_count), 256, 0, stream>>>(
                          static_cast<const T*>(x), c_stride, img_f32, img_u8, pixels)));
+  DK_LAUNCH_CHECK(ctx);
+  return 0;
+}
+
+extern "C" int dk_image_post_masked(dk_ctx* ctx, int dtype, const void* x, int c_stride, const uint8_t* orig,
+                                    const uint8_t* mask, uint8_t* img_u8, long long pixels, void* stream_) {
+  DK_REQUIRE(ctx != nullptr, "dk_image_post_masked: null ctx");
+  DkDeviceGuard dk_guard_(ctx);
+  DK_DTYPE_OK(dtype);
+  DK_REQUIRE(x != nullptr && orig != nullptr && mask != nullptr && img_u8 != nullptr,
+             "dk_image_post_masked: null tensor");
+  DK_REQUIRE(c_stride >= 3, "dk_image_post_masked: c_stride (%d) must be >= 3", c_stride);
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DK_DISPATCH(dtype, (image_post_masked_kernel<T><<<grid_for(pixels * 3, 256, ctx->sm_count), 256, 0, stream>>>(
+                         static_cast<const T*>(x), c_stride, orig, mask, img_u8, pixels)));
+  DK_LAUNCH_CHECK(ctx);
+  return 0;
+}
+
+extern "C" int dk_inpaint_blend(dk_ctx* ctx, const float* x0, const float* noise, const uint8_t* mask, float* x,
+                                long long pixels, int C, float sigma_next, void* stream_) {
+  DK_REQUIRE(ctx != nullptr, "dk_inpaint_blend: null ctx");
+  DkDeviceGuard dk_guard_(ctx);
+  DK_REQUIRE(x0 != nullptr && noise != nullptr && mask != nullptr && x != nullptr, "dk_inpaint_blend: null tensor");
+  DK_REQUIRE(C > 0 && C % 4 == 0, "dk_inpaint_blend: C (%d) must be a positive multiple of 4", C);
+  DK_REQUIRE(((reinterpret_cast<uintptr_t>(x0) | reinterpret_cast<uintptr_t>(noise) | reinterpret_cast<uintptr_t>(x)) &
+              15u) == 0,
+             "dk_inpaint_blend: x0, noise and x must be 16-byte aligned");
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  const int grid = grid_for(pixels * (C / 4), 256, ctx->sm_count);
+  const float4* a = reinterpret_cast<const float4*>(x0);
+  const float4* b = reinterpret_cast<const float4*>(noise);
+  float4* o = reinterpret_cast<float4*>(x);
+  if (C == 16)
+    inpaint_blend_kernel<4><<<grid, 256, 0, stream>>>(a, b, mask, o, pixels, 4, sigma_next);
+  else
+    inpaint_blend_kernel<0><<<grid, 256, 0, stream>>>(a, b, mask, o, pixels, C / 4, sigma_next);
   DK_LAUNCH_CHECK(ctx);
   return 0;
 }

@@ -507,3 +507,34 @@ def image_post(x, want_u8: bool = True):
     c = ctx(x.device.index)
     c.call("dk_image_post", dtype_code(x.dtype), ptr(x), Cp, ptr(f), ptr(u), B * H * W)
     return f, u
+
+
+def _chk_mask(mask, shape, name: str):
+    if mask.dtype != torch.uint8 or not mask.is_cuda or not mask.is_contiguous() or tuple(mask.shape) != tuple(shape):
+        raise _lib.DkError(f"{name}: expected a contiguous CUDA uint8 tensor of shape {tuple(shape)}, got "
+                           f"{mask.dtype} {tuple(mask.shape)} on {mask.device}")
+
+
+def inpaint_blend(x, x0, noise, mask, sigma_next: float):
+    """in place on x: x = mask ? x : sigma_next * noise + (1 - sigma_next) * x0.  x, x0, noise fp32 NHWC [B,H,W,C]
+    (C % 4 == 0); mask uint8 [B,H,W], non-zero = the cell is being regenerated (left untouched)."""
+    for t, n in ((x, "x"), (x0, "x0"), (noise, "noise")):
+        if t.dtype != torch.float32 or not t.is_cuda or not t.is_contiguous() or t.shape != x.shape:
+            raise _lib.DkError(f"inpaint_blend.{n}: expected a contiguous CUDA fp32 tensor of shape {tuple(x.shape)}")
+    _chk_mask(mask, x.shape[:-1], "inpaint_blend.mask")
+    c = ctx(x.device.index)
+    c.call("dk_inpaint_blend", ptr(x0), ptr(noise), ptr(mask), ptr(x), mask.numel(), x.shape[-1], sigma_next)
+    return x
+
+
+def image_post_masked(x, orig, mask):
+    """decoder output NHWC [B,H,W,Cpad] 16-bit, orig uint8 [B,H,W,3], pixel mask uint8 [B,H,W] -> uint8 [B,H,W,3]:
+    image_post's uint8 where the mask is non-zero, orig where it is zero."""
+    _chk16(x, "image_post_masked.x")
+    B, H, W, Cp = x.shape
+    _chk_mask(orig, (B, H, W, 3), "image_post_masked.orig")
+    _chk_mask(mask, (B, H, W), "image_post_masked.mask")
+    u = torch.empty((B, H, W, 3), dtype=torch.uint8, device=x.device)
+    c = ctx(x.device.index)
+    c.call("dk_image_post_masked", dtype_code(x.dtype), ptr(x), Cp, ptr(orig), ptr(mask), ptr(u), B * H * W)
+    return u

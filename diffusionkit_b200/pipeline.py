@@ -12,13 +12,17 @@ Differences that are deliberate (documented in DESIGN.md):
     `conditioning` / `pooled_conditioning` to generate_image or call denoise_latents.
   * img2img (`image_path`, `denoise`): the VAE encoder is built on first use.
   * batch-N extension: `seed` may be a list of ints — one independent image per seed (the reference is batch 1);
-    a scalar seed behaves exactly like the reference.
+    a scalar seed behaves exactly like the reference.  `image_path` may then be a list too, one image per seed.
+  * inpainting extension (`mask_path`, the reference has none): latent-blend inpainting on the img2img flow.  After
+    every Euler step the latent cells outside the mask are reset to sigma_next * noise + (1 - sigma_next) * x_T
+    (dk_inpaint_blend), and generate_image restores the pixels outside the mask from the input image in uint8
+    (dk_image_post_masked).  A call without a mask launches exactly what it did before.
 """
 from __future__ import annotations
 
 import math
 import time
-from typing import Dict, List, Optional, Sequence, Tuple, Union
+from typing import Dict, List, NamedTuple, Optional, Sequence, Tuple, Union
 
 import numpy as np
 import torch
@@ -73,6 +77,108 @@ def _bytes2gigabytes(n: int) -> float:
     return n / 1024 ** 3
 
 
+def _open_image(image, what: str):
+    """a file path, a PIL image or a uint8 array -> PIL image"""
+    from PIL import Image
+
+    if isinstance(image, (str, bytes)) or hasattr(image, "__fspath__"):
+        return Image.open(image)
+    if isinstance(image, np.ndarray):
+        if what == "image" and (image.dtype != np.uint8 or image.ndim != 3 or image.shape[2] < 3):
+            raise ValueError("image array must be uint8 (H, W, >=3)")
+        if what == "mask":
+            if image.ndim == 3 and image.shape[2] == 1:
+                image = image[:, :, 0]
+            if image.dtype != np.uint8 or not (image.ndim == 2 or (image.ndim == 3 and image.shape[2] in (3, 4))):
+                raise ValueError("mask array must be uint8 (H, W), (H, W, 1), (H, W, 3) or (H, W, 4)")
+            return Image.fromarray(image)
+        return Image.fromarray(image[:, :, :3])
+    return image
+
+
+def load_image_u8(image) -> Tuple[np.ndarray, Tuple[int, int]]:
+    """read_image's resize rule (reference mlx/__init__.py:540-546) -> (uint8 (H, W, >=3) with H, W the original size
+    cut down to multiples of 64 by a LANCZOS resize, original (width, height))"""
+    from PIL import Image
+
+    image = _open_image(image, "image")
+    size = (image.width, image.height)
+    W, H = (dim - dim % 64 for dim in size)
+    if W == 0 or H == 0:
+        raise ValueError(f"image {image.width}x{image.height} is smaller than 64x64")
+    if W != image.width or H != image.height:
+        image = image.resize((W, H), Image.LANCZOS)
+    arr = np.asarray(image)
+    if arr.ndim == 2:
+        raise ValueError("greyscale images are not supported (the reference indexes img[:, :, :3])")
+    return np.ascontiguousarray(arr), size
+
+
+def prepare_inpaint_mask(mask, image_size: Tuple[int, int]) -> Tuple[np.ndarray, np.ndarray]:
+    """Inpainting mask (a path, a PIL image or a uint8 array) -> (pixel mask p (H, W), latent mask m (H/8, W/8)), both
+    uint8 in {0, 1}; 1 = regenerate.  image_size = (width, height) of the image the mask belongs to BEFORE read_image's
+    resize; the mask must have that size and is resized with NEAREST to the image's target size.
+      p = greyscale(mask) >= 128 (white = regenerate);  m[y, x] = any(p[8y:8y+8, 8x:8x+8])
+    so a latent cell that touches any repainted pixel is repainted and thin strokes survive the 8x downsampling."""
+    from PIL import Image
+
+    mask = _open_image(mask, "mask")
+    if (mask.width, mask.height) != tuple(image_size):
+        raise ValueError(f"mask is {mask.width}x{mask.height}, its image is {image_size[0]}x{image_size[1]}: "
+                         "they must have the same original size")
+    W, H = (dim - dim % 64 for dim in image_size)
+    mask = mask.convert("L")
+    if (W, H) != tuple(image_size):
+        mask = mask.resize((W, H), Image.NEAREST)
+    p = (np.asarray(mask) >= 128).astype(np.uint8)
+    m = p.reshape(H // 8, 8, W // 8, 8).max(axis=(1, 3))
+    return p, np.ascontiguousarray(m)
+
+
+class ImageInputs(NamedTuple):
+    """Host-side inputs of an img2img / inpainting call, prepared by prepare_image_inputs."""
+    images: np.ndarray                   # (1 or B, H, W, >=3) uint8, resized; one entry is shared by every seed
+    pixel_mask: Optional[np.ndarray]     # (B, H, W) uint8 or None (plain img2img)
+    latent_mask: Optional[np.ndarray]    # (B, H/8, W/8) uint8 or None
+
+
+def prepare_image_inputs(image_path, mask_path, n: int) -> Optional[ImageInputs]:
+    """image_path / mask_path: one image (or mask) shared by all n seeds, or a list with one entry per seed; every
+    image must resize to the same size and every mask must have its image's original size.  None without an image."""
+    if image_path is None:
+        if mask_path is not None:
+            raise ValueError("mask_path needs an image_path: inpainting regenerates part of an input image")
+        return None
+
+    def per_seed(v, name):
+        if not isinstance(v, (list, tuple)):
+            return None
+        if len(v) != n:
+            raise ValueError(f"{name} is a list of {len(v)} entries for {n} seed(s): give one per seed, or one shared")
+        return list(v)
+
+    images = per_seed(image_path, "image_path")
+    loaded = [load_image_u8(im) for im in (images if images is not None else [image_path])]
+    if len({a.shape[:2] for a, _ in loaded}) > 1:
+        raise ValueError("the images of a list resize to different sizes "
+                         f"{sorted({a.shape[:2] for a, _ in loaded})}: a batch needs one latent size")
+    if len(loaded) == 1:
+        arr = loaded[0][0][None]                                  # as the single-image img2img path always was
+    else:
+        arr = np.stack([a[:, :, :3] for a, _ in loaded])
+    if mask_path is None:
+        return ImageInputs(arr, None, None)
+    masks = per_seed(mask_path, "mask_path")
+    sizes = [s for _, s in loaded]
+    if masks is None:
+        prepared = [prepare_inpaint_mask(mask_path, s) for s in sizes]
+    else:
+        prepared = [prepare_inpaint_mask(mk, sizes[i if len(sizes) > 1 else 0]) for i, mk in enumerate(masks)]
+    if len(prepared) == 1:
+        prepared = prepared * n
+    return ImageInputs(arr, np.stack([p for p, _ in prepared]), np.stack([m for _, m in prepared]))
+
+
 class CFGDenoiser:
     """Helper for applying CFG scaling to diffusion outputs (reference mlx/__init__.py:674-719).
     x_t is the fp32 sampler state on the device; one call = prepare (cast / CFG doubling) + MMDiT forward; the
@@ -100,7 +206,9 @@ class CFGDenoiser:
 
 def sample_euler(model: CFGDenoiser, x, sigmas, extra_args=None):
     """Implements Algorithm 2 (Euler steps) from Karras et al. (2022) — reference mlx/__init__.py:761-788.
-    x: (B, H, W, 16) fp32 device tensor (updated in place); sigmas: 1-D float32 numpy/torch array."""
+    x: (B, H, W, 16) fp32 device tensor (updated in place); sigmas: 1-D float32 numpy/torch array.
+    extra_args["inpaint"] (optional, an extension): (x0, noise, latent mask) of a masked img2img run; after every step
+    the kept cells (mask 0) are set to sigma_next * noise + (1 - sigma_next) * x0 (dk_inpaint_blend)."""
     extra_args = {} if extra_args is None else dict(extra_args)
     pipe = model.model
     sig = np.asarray(sigmas, dtype=np.float32)
@@ -108,6 +216,7 @@ def sample_euler(model: CFGDenoiser, x, sigmas, extra_args=None):
     timesteps = torch.from_numpy(np.asarray(pipe.sampler.timestep(sig), dtype=np.float32)).to(
         pipe.activation_dtype).to(torch.float32).tolist()
     pooled = extra_args.pop("pooled_conditioning")
+    inpaint = extra_args.pop("inpaint", None)
     model.cache_modulation_params(pooled, timesteps)
     cfg_weight = float(extra_args.get("cfg_weight", 0.0))
     conditioning = extra_args["conditioning"]
@@ -117,6 +226,8 @@ def sample_euler(model: CFGDenoiser, x, sigmas, extra_args=None):
         xin, out = model(x, timesteps[i], float(sig[i]), conditioning, cfg_weight)
         # denoised = xin - out * sigma; CFG mix; d = (x - denoised) / sigma; x += d * (sigma_next - sigma)
         ops.sampler_step(x, xin, out, float(sig[i]), float(sig[i + 1]), cfg_weight)
+        if inpaint is not None:
+            ops.inpaint_blend(x, *inpaint, float(sig[i + 1]))
         events[i + 1].record()
     model.clear_cache()
     torch.cuda.current_stream().synchronize()  # the reference syncs every step (mx.eval, :782); once is enough here
@@ -363,17 +474,29 @@ class DiffusionPipeline:
         seed=None,
         image_path: Optional[str] = None,
         denoise: float = 1.0,
+        mask_path=None,
         *,
         noise: Optional[torch.Tensor] = None,
     ):
         """-> (latent NHWC (B, H, W, 16) fp32 on the device, iter_time list).  `noise` (optional, device fp32
         (B, H, W, 16)) replaces the host-side numpy draw of get_noise for callers whose inputs already live in HBM.
         `image_path` (img2img): a file path, a PIL image or a uint8 HWC array; the latent size then follows the image
-        (the reference ignores latent_size in that case too, :273)."""
+        (the reference ignores latent_size in that case too, :273).  A list gives one image per seed (all must resize
+        to the same size); a single image is shared by every seed.
+        `mask_path` (inpainting, an extension): same kinds of value as `image_path`, one shared or a list with one per
+        seed, at the original size of its image; white (>= 128) = regenerate.  Latent cells outside the mask follow the
+        image's noised trajectory after every step and end exactly at its encoding (prepare_inpaint_mask)."""
         if image_path is None:
             denoise = 1.0                                                   # :270-271
         elif not (0.0 <= denoise <= 1.0):
             raise ValueError(f"denoise must be in [0, 1], got {denoise}")
+        n = len(seed) if isinstance(seed, (list, tuple)) else 1
+        src = prepare_image_inputs(image_path, mask_path, n)
+        return self._denoise_latents(conditioning, pooled_conditioning, num_steps, cfg_weight, latent_size, seed, src,
+                                     denoise, noise)
+
+    def _denoise_latents(self, conditioning, pooled_conditioning, num_steps, cfg_weight, latent_size, seed,
+                         src: Optional[ImageInputs], denoise, noise):
         seeds: List[int]
         if seed is None:
             seeds = [int(time.time())]
@@ -399,8 +522,8 @@ class DiffusionPipeline:
                 f"({'[positive | negative] x ' if reps == 2 else ''}{B} image(s)) for cfg_weight={cfg_weight}")
 
         hidden = None
-        if image_path is not None:
-            hidden = self._encode_image_hidden(image_path)                  # (1, H, W, 32) = (mean | logvar)
+        if src is not None:
+            hidden = self._encode_u8(src.images)                            # (1 or B, H, W, 32) = (mean | logvar)
             H, W = hidden.shape[1], hidden.shape[2]
         x_T = self.get_empty_latent(H, W)                                   # (1, H, W, 16) host
         if noise is None:
@@ -420,11 +543,17 @@ class DiffusionPipeline:
             noise = noise.to(self.device, dtype=torch.float32, non_blocking=True).contiguous()
             lf = self.latent_format
             x_T = torch.empty_like(noise)
-            for b in range(B):
-                ops.vae_sample_latent(hidden, noise[b:b + 1], lf.shift_factor, lf.scale_factor, out=x_T[b:b + 1])
+            if hidden.shape[0] == B:                                        # one image per seed: one launch
+                ops.vae_sample_latent(hidden, noise, lf.shift_factor, lf.scale_factor, out=x_T)
+            else:                                                           # one image shared by every seed
+                for b in range(B):
+                    ops.vae_sample_latent(hidden, noise[b:b + 1], lf.shift_factor, lf.scale_factor, out=x_T[b:b + 1])
             x = ops.axpby(noise, x_T, s0, 1.0 - s0)
         extra_args = {"conditioning": conditioning, "cfg_weight": cfg_weight,
                       "pooled_conditioning": pooled_conditioning}
+        if src is not None and src.latent_mask is not None:
+            mask = torch.from_numpy(src.latent_mask).pin_memory().to(self.device, non_blocking=True)
+            extra_args["inpaint"] = (x_T, noise, mask)
         latent, iter_time = sample_euler(CFGDenoiser(self), x, sigmas, extra_args=extra_args)
         latent = ops.axpb(latent, 1.0 / self.latent_format.scale_factor, self.latent_format.shift_factor)  # process_out
         return latent, iter_time
@@ -441,12 +570,18 @@ class DiffusionPipeline:
         verbose: bool = True,
         image_path: Optional[str] = None,
         denoise: float = 1.0,
+        mask_path=None,
         *,
         conditioning=None,
         pooled_conditioning=None,
     ):
+        """With `mask_path` (inpainting, see denoise_latents) the decoded image is composited in uint8: pixels outside
+        the mask are the resized input image, bit for bit."""
         assert latent_size[0] % 2 == 0, f"Height must be divisible by 16 ({latent_size[0]*8}/16={latent_size[0]/2})"
         assert latent_size[1] % 2 == 0, f"Width must be divisible by 16 ({latent_size[1]*8}/16={latent_size[1]/2})"
+        if image_path is not None and not (0.0 <= denoise <= 1.0):
+            raise ValueError(f"denoise must be in [0, 1], got {denoise}")
+        src = prepare_image_inputs(image_path, mask_path, len(seed) if isinstance(seed, (list, tuple)) else 1)
         self.check_and_load_models()
         start_time = time.time()
 
@@ -472,9 +607,8 @@ class DiffusionPipeline:
         torch.cuda.reset_peak_memory_stats(self.device)
         t0 = time.time()
         log["denoising"]["pre"] = mem()
-        latents, iter_time = self.denoise_latents(conditioning, pooled_conditioning, num_steps=num_steps,
-                                                  cfg_weight=cfg_weight, latent_size=latent_size, seed=seed,
-                                                  image_path=image_path, denoise=denoise)
+        latents, iter_time = self._denoise_latents(conditioning, pooled_conditioning, num_steps, cfg_weight,
+                                                   latent_size, seed, src, denoise if src is not None else 1.0, None)
         torch.cuda.synchronize(self.device)
         log["denoising"]["post"] = mem()
         log["denoising"]["time"] = round(time.time() - t0, 3)
@@ -485,7 +619,10 @@ class DiffusionPipeline:
         t0 = time.time()
         log["decoding"]["pre"] = mem()
         latents16 = ops.cast_to_16(latents, self.activation_dtype)          # latents.astype(activation_dtype) (:459)
-        _, u8 = self._decode(latents16, want_u8=True)
+        if src is not None and src.pixel_mask is not None:
+            u8 = self._decode_composite(latents16, src)
+        else:
+            _, u8 = self._decode(latents16, want_u8=True)
         host = getattr(self, "_host_u8", None)                              # pinned staging, reused across calls
         if host is None or host.shape != u8.shape:
             host = self._host_u8 = torch.empty(u8.shape, dtype=torch.uint8, pin_memory=True)
@@ -535,23 +672,7 @@ class DiffusionPipeline:
 
     def _load_image_u8(self, image) -> np.ndarray:
         """-> uint8 (H, W, >=3) with H, W multiples of 64 (read_image's resize rule, :540-546)"""
-        from PIL import Image
-
-        if isinstance(image, (str, bytes)) or hasattr(image, "__fspath__"):
-            image = Image.open(image)
-        if isinstance(image, np.ndarray):
-            if image.dtype != np.uint8 or image.ndim != 3 or image.shape[2] < 3:
-                raise ValueError("image array must be uint8 (H, W, >=3)")
-            image = Image.fromarray(image[:, :, :3])
-        W, H = (dim - dim % 64 for dim in (image.width, image.height))
-        if W == 0 or H == 0:
-            raise ValueError(f"image {image.width}x{image.height} is smaller than 64x64")
-        if W != image.width or H != image.height:
-            image = image.resize((W, H), Image.LANCZOS)
-        arr = np.asarray(image)
-        if arr.ndim == 2:
-            raise ValueError("greyscale images are not supported (the reference indexes img[:, :, :3])")
-        return np.ascontiguousarray(arr)
+        return load_image_u8(image)[0]
 
     def read_image(self, image_path):
         """-> (1, H, W, 3) float32 in [-1, 1] on the host (reference :536-551)"""
@@ -559,10 +680,13 @@ class DiffusionPipeline:
         return (torch.from_numpy(arr[:, :, :3].astype(np.float32)) / 255 * 2 - 1.0).unsqueeze(0)
 
     def _encode_image_hidden(self, image_path) -> torch.Tensor:
+        return self._encode_u8(self._load_image_u8(image_path)[None])
+
+    def _encode_u8(self, arr: np.ndarray) -> torch.Tensor:
+        """uint8 (N, H, W, >=3) resized images -> encoder hidden (N, H/8, W/8, 32), one encoder run at batch N"""
         if not hasattr(self, "encoder"):
             self.load_encoder()
-        arr = self._load_image_u8(image_path)
-        host = torch.from_numpy(arr).unsqueeze(0).pin_memory()
+        host = torch.from_numpy(arr).pin_memory()
         return self.encoder(host.to(self.device, non_blocking=True))       # the /255*2-1 runs in dk_image_pre
 
     def encode_image_to_latents(self, image_path, seed):
@@ -585,6 +709,16 @@ class DiffusionPipeline:
         B, Ho, Wo, _ = x.shape
         padded = x.as_strided((B, Ho, Wo, x.stride(2)), (x.stride(0), x.stride(1), x.stride(2), 1))
         return ops.image_post(padded, want_u8=want_u8)
+
+    def _decode_composite(self, x_t, src: ImageInputs) -> torch.Tensor:
+        """decode, then uint8 = pixel mask ? decoded : resized input image  (inpainting)"""
+        x = self.decoder(x_t)
+        B, Ho, Wo, _ = x.shape
+        padded = x.as_strided((B, Ho, Wo, x.stride(2)), (x.stride(0), x.stride(1), x.stride(2), 1))
+        orig = np.ascontiguousarray(np.broadcast_to(src.images[:, :, :, :3], (B, Ho, Wo, 3)))
+        orig = torch.from_numpy(orig).pin_memory().to(self.device, non_blocking=True)
+        mask = torch.from_numpy(src.pixel_mask).pin_memory().to(self.device, non_blocking=True)
+        return ops.image_post_masked(padded, orig, mask)
 
     def decode_latents_to_image(self, x_t):
         """x = decoder(x_t); clip(x / 2 + 0.5, 0, 1)  (:581-584) -> (B, 8H, 8W, 3) float in [0, 1]"""

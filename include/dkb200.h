@@ -266,6 +266,22 @@ int dk_image_post(dk_ctx* ctx, int dtype, const void* x, int c_stride, float* im
                   void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * masked img2img (inpainting).  No reference counterpart: the reference has no inpainting.  These compose with its
+ * img2img flow: noise_scaling (sampler.py:41-42), the Euler step (__init__.py:779-781) and the decode tail
+ * (__init__.py:583, :526).
+ * ------------------------------------------------------------------------------------------- */
+/* after an Euler step to sigma_next, re-noise the kept latent cells to the image's trajectory:
+ * x = mask ? x : sigma_next * noise + (1 - sigma_next) * x0   (fp32; x0 = process_in of the posterior sample)
+ * x0, noise, x [pixels, C] (C % 4 == 0, 16-byte aligned); mask one byte per latent pixel, non-zero = regenerate:
+ * those cells of x are left untouched */
+int dk_inpaint_blend(dk_ctx* ctx, const float* x0, const float* noise, const uint8_t* mask, float* x, long long pixels,
+                     int C, float sigma_next, void* stream);
+/* inpainting composite: img_u8 = mask ? dk_image_post's uint8 (bit-identical) : orig
+ * x NHWC [.., c_stride] 16-bit decoder output, orig [pixels, 3] uint8, mask one byte per pixel (non-zero = decoded) */
+int dk_image_post_masked(dk_ctx* ctx, int dtype, const void* x, int c_stride, const uint8_t* orig, const uint8_t* mask,
+                         uint8_t* img_u8, long long pixels, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * one-time weight broadcast for multi-GPU batch sharding (no per-step collective).
  * The Python host uses torch.distributed (NCCL) for the rendezvous; these are thin NCCL wrappers
  * for hosts without torch.
