@@ -9,6 +9,7 @@ DiffusionPipeline / FluxPipeline API (reference: argmaxinc/DiffusionKit, python/
 """
 from ._lib import DkError  # noqa: F401
 from .config import FLUX_DEV, FLUX_SCHNELL, SD3_2b, SD3_8b, MMDiTConfig, VAEDecoderConfig, VAEEncoderConfig  # noqa: F401
+from .lora import LoraInfo  # noqa: F401
 from .mmdit import MMDiT  # noqa: F401
 from .pipeline import (CFGDenoiser, DiffusionPipeline, FluxLatentFormat, FluxPipeline, LatentFormat,  # noqa: F401
                        SD3LatentFormat, sample_euler)

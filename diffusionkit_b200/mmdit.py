@@ -81,6 +81,10 @@ class MMDiT:
                 t = t.to(device=dev, dtype=dt)
             return t.contiguous()
 
+        # reference weight name -> the tensor or window of a packed buffer holding it (2-D [out, in]); in-place
+        # weight edits (lora.py) go through these views so captured graphs keep their pointers
+        views: Dict[str, torch.Tensor] = {}
+        self.weight_views = views
         self.w_x = get("x_embedder.proj.weight").reshape(h, -1).contiguous()          # (h, 64)
         self.b_x = get("x_embedder.proj.bias")
         self.pos_table = get("x_pos_embedder.pos_embed.weight") if "x_pos_embedder.pos_embed.weight" in P else None
@@ -90,13 +94,19 @@ class MMDiT:
         self.t2 = (get("t_embedder.mlp.layers.2.weight"), get("t_embedder.mlp.layers.2.bias"))
         self.w_ctx, self.b_ctx = get("context_embedder.weight"), get("context_embedder.bias")
         self.w_final, self.b_final = get("final_layer.linear.weight"), get("final_layer.linear.bias")
+        views["x_embedder.proj.weight"] = self.w_x
+        for name, w in (("y_embedder.mlp.layers.0", self.y0[0]), ("y_embedder.mlp.layers.2", self.y2[0]),
+                        ("t_embedder.mlp.layers.0", self.t0[0]), ("t_embedder.mlp.layers.2", self.t2[0]),
+                        ("context_embedder", self.w_ctx), ("final_layer.linear", self.w_final)):
+            views[name + ".weight"] = w
 
-        mod_w, mod_b = [], []
+        mod_w, mod_b, mod_rows = [], [], {}
         self.mod_total = 0
 
         def add_mod(prefix) -> int:
             off = self.mod_total
             w = get(prefix + ".adaLN_modulation.layers.1.weight")
+            mod_rows[prefix + ".adaLN_modulation.layers.1.weight"] = (off, off + w.shape[0])
             mod_w.append(w)
             mod_b.append(get(prefix + ".adaLN_modulation.layers.1.bias"))
             self.mod_total += w.shape[0]
@@ -109,6 +119,8 @@ class MMDiT:
             wq, wk, wv = get(prefix + ".attn.q_proj.weight"), get(prefix + ".attn.k_proj.weight"), get(
                 prefix + ".attn.v_proj.weight")
             s.w_qkv = torch.cat([wq, wk, wv], dim=0).contiguous()
+            for j, n in enumerate("qkv"):
+                views[f"{prefix}.attn.{n}_proj.weight"] = s.w_qkv[j * h:(j + 1) * h]
             bq, bv = get(prefix + ".attn.q_proj.bias"), get(prefix + ".attn.v_proj.bias")
             s.b_qkv = torch.cat([bq, torch.zeros_like(bq), bv]).contiguous()          # no k bias (quirk Q3)
             s.w_o = s.b_o = s.w_fc1 = s.b_fc1 = s.w_fc2 = s.b_fc2 = s.w_out = None
@@ -119,9 +131,14 @@ class MMDiT:
                     # u += gate * ([attn | gelu(fc1)] @ [Wo | W2]^T + bo); fc2.bias is zeroed (mmdit.py:742)
                     s.w_out = torch.cat([get(prefix + ".attn.o_proj.weight"), get(prefix + ".mlp.fc2.weight")],
                                         dim=1).contiguous()
+                    views[prefix + ".attn.o_proj.weight"] = s.w_out[:, :h]
+                    views[prefix + ".mlp.fc2.weight"] = s.w_out[:, h:]
                 else:
                     s.w_o = get(prefix + ".attn.o_proj.weight")
                     s.w_fc2, s.b_fc2 = get(prefix + ".mlp.fc2.weight"), get(prefix + ".mlp.fc2.bias")
+                    views[prefix + ".attn.o_proj.weight"] = s.w_o
+                    views[prefix + ".mlp.fc2.weight"] = s.w_fc2
+                views[prefix + ".mlp.fc1.weight"] = s.w_fc1
             s.q_norm = s.k_norm = None
             if c.use_qk_norm:
                 s.q_norm = get(prefix + ".qk_norm.q_norm.weight")
@@ -144,6 +161,8 @@ class MMDiT:
         self.final_mod_off = add_mod("final_layer")
         self.w_mod = torch.cat(mod_w, dim=0).contiguous()                             # (mod_total, h)
         self.b_mod = torch.cat(mod_b, dim=0).contiguous()
+        for name, (r0, r1) in mod_rows.items():
+            views[name] = self.w_mod[r0:r1]
 
     # ------------------------------------------------------------------------------------------ modulation cache
     def timestep_embedding(self, t: torch.Tensor) -> torch.Tensor:
@@ -184,6 +203,12 @@ class MMDiT:
 
     def clear_modulation_params_cache(self):
         self._mod_index, self._mod_all = {}, None
+
+    def invalidate_modulation_cache(self):
+        """after a weight edit: drop the cached rows AND the current timestep, so a forward without a fresh
+        cache_modulation_params raises KeyError instead of reusing rows of the old adaLN weights"""
+        self.clear_modulation_params_cache()
+        self._cur_t = None
 
     def select_timestep(self, timestep: float):
         """Make `timestep`'s modulation rows current (one D2D copy; keeps the forward timestep-invariant)."""

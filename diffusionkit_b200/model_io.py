@@ -29,8 +29,141 @@ def _conv_oihw_to_ohwi(w: Tensor) -> Tensor:
     return w.permute(0, 2, 3, 1).contiguous()
 
 
-# ------------------------------------------------------------------------------------------------ FLUX (BFL layout)
+# ------------------------------------------------------------------------------------------------ Linear routing
+# An upstream Linear module -> the reference Linear modules its weight is split into:
+#   (split dim, ((reference module, width in units), ...))
+# dim 0 splits the weight's rows (output features), dim 1 its columns (input features); the widths are in units of
+# size / sum(units).  One table serves both the checkpoint converters below and the LoRA converter (lora_to_params), so
+# a split rule cannot differ between a base weight and an adapter on it.
+Route = Tuple[int, Tuple[Tuple[str, int], ...]]
+
 _FLUX_STREAM = {"img": "image_transformer_block", "txt": "text_transformer_block"}
+_FLUX_FIXED = {
+    "img_in": "x_embedder.proj", "txt_in": "context_embedder",
+    "time_in.in_layer": "t_embedder.mlp.layers.0", "time_in.out_layer": "t_embedder.mlp.layers.2",
+    "vector_in.in_layer": "y_embedder.mlp.layers.0", "vector_in.out_layer": "y_embedder.mlp.layers.2",
+    "final_layer.linear": "final_layer.linear", "final_layer.adaLN_modulation.1": "final_layer.adaLN_modulation.layers.1",
+}
+_SD3_FIXED = {
+    "context_embedder": "context_embedder", "final_layer.linear": "final_layer.linear",
+    "final_layer.adaLN_modulation.1": "final_layer.adaLN_modulation.layers.1",
+    "t_embedder.mlp.0": "t_embedder.mlp.layers.0", "t_embedder.mlp.2": "t_embedder.mlp.layers.2",
+    "y_embedder.mlp.0": "y_embedder.mlp.layers.0", "y_embedder.mlp.2": "y_embedder.mlp.layers.2",
+}
+_BLOCK_PARTS = {"qkv": ("attn.q_proj", "attn.k_proj", "attn.v_proj"), "proj": ("attn.o_proj",),
+                "fc1": ("mlp.fc1",), "fc2": ("mlp.fc2",), "mod": ("adaLN_modulation.layers.1",)}
+
+
+def _block_route(base: str, part: str) -> Route:
+    return 0, tuple((f"{base}.{n}", 1) for n in _BLOCK_PARTS[part])
+
+
+def flux_linear_route(module: str, mlp_ratio: int = 4) -> Optional[Route]:
+    """BFL FLUX Linear module name (no `.weight`) -> Route, or None if `module` is not one of the model's Linears.
+      double_blocks.i.{img,txt}_attn.qkv -> rows [h, h, h] of {q,k,v}_proj;  _attn.proj / _mlp.{0,2} / _mod.lin -> 1:1
+      single_blocks.i.linear1 -> rows [h, h, h, r*h] of {q,k,v}_proj, mlp.fc1
+      single_blocks.i.linear2 -> cols [h, r*h] of o_proj, mlp.fc2;  single_blocks.i.modulation.lin -> 1:1
+      img_in / txt_in / time_in / vector_in / final_layer.* -> embedders / final layer"""
+    m = re.fullmatch(r"double_blocks\.(\d+)\.(img|txt)_(attn\.qkv|attn\.proj|mlp\.0|mlp\.2|mod\.lin)", module)
+    if m:
+        i, stream, part = m.groups()
+        part = {"attn.qkv": "qkv", "attn.proj": "proj", "mlp.0": "fc1", "mlp.2": "fc2", "mod.lin": "mod"}[part]
+        return _block_route(f"multimodal_transformer_blocks.{i}.{_FLUX_STREAM[stream]}", part)
+    m = re.fullmatch(r"single_blocks\.(\d+)\.(linear1|linear2|modulation\.lin)", module)
+    if m:
+        i, part = m.groups()
+        base = f"unified_transformer_blocks.{i}.transformer_block"
+        if part == "linear1":
+            return 0, tuple((f"{base}.{n}", w) for n, w in
+                            (("attn.q_proj", 1), ("attn.k_proj", 1), ("attn.v_proj", 1), ("mlp.fc1", mlp_ratio)))
+        if part == "linear2":
+            return 1, ((f"{base}.attn.o_proj", 1), (f"{base}.mlp.fc2", mlp_ratio))
+        return _block_route(base, "mod")
+    if module in _FLUX_FIXED:
+        return 0, ((_FLUX_FIXED[module], 1),)
+    return None
+
+
+def sd3_linear_route(module: str) -> Optional[Route]:
+    """Stability SD3 / SD3.5 Linear module name (no `model.diffusion_model.` prefix, no `.weight`) -> Route or None.
+      joint_blocks.i.{x_block,context_block}.attn.qkv -> rows [h, h, h] of {q,k,v}_proj;  attn.proj, mlp.fc1,
+      mlp.fc2, adaLN_modulation.1 -> 1:1;  context_embedder, {t,y}_embedder.mlp.{0,2}, final_layer.* -> 1:1.
+    x_embedder.proj is a 2x2 conv, not a Linear."""
+    m = re.fullmatch(r"joint_blocks\.(\d+)\.(context_block|x_block)\.(attn\.qkv|attn\.proj|mlp\.fc1|mlp\.fc2|"
+                     r"adaLN_modulation\.1)", module)
+    if m:
+        i, blk, part = m.groups()
+        stream = "text_transformer_block" if blk == "context_block" else "image_transformer_block"
+        part = {"attn.qkv": "qkv", "attn.proj": "proj", "mlp.fc1": "fc1", "mlp.fc2": "fc2",
+                "adaLN_modulation.1": "mod"}[part]
+        return _block_route(f"multimodal_transformer_blocks.{i}.{stream}", part)
+    if module in _SD3_FIXED:
+        return 0, ((_SD3_FIXED[module], 1),)
+    return None
+
+
+def flux_linear_modules(depth_multimodal: int, depth_unified: int) -> List[str]:
+    """every upstream Linear module of a FLUX model with these depths (the names flux_linear_route accepts)"""
+    mods = list(_FLUX_FIXED)
+    for i in range(depth_multimodal):
+        for s in _FLUX_STREAM:
+            mods += [f"double_blocks.{i}.{s}_{p}" for p in ("attn.qkv", "attn.proj", "mlp.0", "mlp.2", "mod.lin")]
+    for i in range(depth_unified):
+        mods += [f"single_blocks.{i}.{p}" for p in ("linear1", "linear2", "modulation.lin")]
+    return mods
+
+
+def sd3_linear_modules(depth_multimodal: int) -> List[str]:
+    """every upstream Linear module of an SD3 / SD3.5 model with this depth; the last context block stops after its
+    qkv projection (reference mmdit.py:62-66), so it has no attn.proj / mlp"""
+    mods = list(_SD3_FIXED)
+    for i in range(depth_multimodal):
+        for blk in ("x_block", "context_block"):
+            last_ctx = blk == "context_block" and i == depth_multimodal - 1
+            parts = ("attn.qkv", "adaLN_modulation.1") if last_ctx else (
+                "attn.qkv", "attn.proj", "mlp.fc1", "mlp.fc2", "adaLN_modulation.1")
+            mods += [f"joint_blocks.{i}.{blk}.{p}" for p in parts]
+    return mods
+
+
+def _split_sizes(n: int, parts, what: str) -> List[int]:
+    units = sum(w for _, w in parts)
+    if n % units:
+        raise ValueError(f"{what}: size {n} does not split into {[name for name, _ in parts]} ({units} equal units)")
+    return [n // units * w for _, w in parts]
+
+
+def _convert_linear(route: Route, leaf: str, v: Tensor, out: Dict[str, Tensor], what: str) -> None:
+    """one upstream Linear tensor (`leaf` = weight / bias) -> its reference tensors in `out`"""
+    dim, parts = route
+    if len(parts) == 1:
+        out[f"{parts[0][0]}.{leaf}"] = v
+        return
+    if leaf == "bias" and dim == 1:
+        chunks = [v] * len(parts)            # a column split keeps ONE bias: the reference gives it to every part
+    else:
+        chunks = [c.contiguous() for c in torch.split(v, _split_sizes(v.shape[dim], parts, what), dim=dim)]
+    for (name, _), c in zip(parts, chunks):
+        if leaf == "bias" and name.endswith(".attn.k_proj"):
+            continue                         # no K-projection bias (quirk Q3)
+        out[f"{name}.{leaf}"] = c
+
+
+def lora_to_params(route: Route, A: Tensor, B: Tensor, what: str = "lora") -> List[Tuple[str, Tensor, Tensor]]:
+    """a LoRA pair on one upstream Linear (A = down [r, in], B = up [out, r]; delta = B @ A) -> one
+    (reference weight name, A, B) per reference weight: a row split slices B by rows, a column split slices A by
+    columns, with the same widths the checkpoint converters use for the base weight"""
+    dim, parts = route
+    if len(parts) == 1:
+        return [(parts[0][0] + ".weight", A, B)]
+    if dim == 0:
+        return [(name + ".weight", A, b) for (name, _), b in
+                zip(parts, torch.split(B, _split_sizes(B.shape[0], parts, what), dim=0))]
+    return [(name + ".weight", a, B) for (name, _), a in
+            zip(parts, torch.split(A, _split_sizes(A.shape[1], parts, what), dim=1))]
+
+
+# ------------------------------------------------------------------------------------------------ FLUX (BFL layout)
 
 
 def flux_checkpoint_to_params(sd: Dict[str, Tensor], hidden_size: int = 3072, mlp_ratio: int = 4) -> Dict[str, Tensor]:
@@ -45,77 +178,24 @@ def flux_checkpoint_to_params(sd: Dict[str, Tensor], hidden_size: int = 3072, ml
     single_blocks.i.linear2.weight            -> split cols [h, r*h]       -> attn.o_proj.weight, mlp.fc2.weight
     single_blocks.i.linear2.bias              -> attn.o_proj.bias (and mlp.fc2.bias, which the forward zeroes, mmdit.py:742)
     img_in / txt_in / time_in / vector_in / final_layer.adaLN_modulation.1 -> embedders / final layer
-    The K-projection bias is dropped (quirk Q3) and guidance_in.* is ignored (quirk Q1).
+    The K-projection bias is dropped (quirk Q3) and guidance_in.* is ignored (quirk Q1).  The Linear splits come from
+    flux_linear_route; `hidden_size` is implied by the tensor sizes and kept for existing callers.
     """
-    h = hidden_size
     out: Dict[str, Tensor] = {}
     for key, v in sd.items():
-        m = re.fullmatch(r"double_blocks\.(\d+)\.(img|txt)_(attn|mlp|mod)\.(.+)", key)
-        if m:
-            i, stream, part, rest = m.groups()
-            base = f"multimodal_transformer_blocks.{i}.{_FLUX_STREAM[stream]}"
-            if part == "attn":
-                if rest.startswith("qkv."):
-                    leaf = rest[4:]
-                    for name, chunk in zip("qkv", v.chunk(3, dim=0)):
-                        if name == "k" and leaf == "bias":
-                            continue
-                        out[f"{base}.attn.{name}_proj.{leaf}"] = chunk.contiguous()
-                elif rest.startswith("proj."):
-                    out[f"{base}.attn.o_proj.{rest[5:]}"] = v
-                elif rest == "norm.query_norm.scale":
-                    out[f"{base}.qk_norm.q_norm.weight"] = v
-                elif rest == "norm.key_norm.scale":
-                    out[f"{base}.qk_norm.k_norm.weight"] = v
-                else:
-                    raise KeyError(f"unrecognised FLUX key {key}")
-            elif part == "mlp":
-                idx, leaf = rest.split(".", 1)
-                out[f"{base}.mlp.{'fc1' if idx == '0' else 'fc2'}.{leaf}"] = v
-            else:  # mod.lin.{weight,bias}
-                out[f"{base}.adaLN_modulation.layers.1.{rest.split('.', 1)[1]}"] = v
+        module, _, leaf = key.rpartition(".")
+        route = flux_linear_route(module, mlp_ratio) if leaf in ("weight", "bias") else None
+        if route is not None:
+            if module == "img_in" and leaf == "weight":
+                v = v.reshape(v.shape[0], 1, 1, v.shape[1]).contiguous()    # patchify-as-reshape conv weight
+            _convert_linear(route, leaf, v, out, key)
             continue
-        m = re.fullmatch(r"single_blocks\.(\d+)\.(.+)", key)
+        m = re.fullmatch(r"(double_blocks\.(\d+)\.(img|txt)_attn|single_blocks\.(\d+))\.norm\.(query|key)_norm\.scale", key)
         if m:
-            i, rest = m.groups()
-            base = f"unified_transformer_blocks.{i}.transformer_block"
-            if rest.startswith("linear1."):
-                leaf = rest[8:]
-                q, k, vv, fc1 = torch.split(v, [h, h, h, mlp_ratio * h], dim=0)
-                out[f"{base}.attn.q_proj.{leaf}"] = q.contiguous()
-                if leaf != "bias":
-                    out[f"{base}.attn.k_proj.{leaf}"] = k.contiguous()
-                out[f"{base}.attn.v_proj.{leaf}"] = vv.contiguous()
-                out[f"{base}.mlp.fc1.{leaf}"] = fc1.contiguous()
-            elif rest == "linear2.weight":
-                o, fc2 = torch.split(v, [h, mlp_ratio * h], dim=1)
-                out[f"{base}.attn.o_proj.weight"] = o.contiguous()
-                out[f"{base}.mlp.fc2.weight"] = fc2.contiguous()
-            elif rest == "linear2.bias":
-                out[f"{base}.attn.o_proj.bias"] = v
-                out[f"{base}.mlp.fc2.bias"] = v
-            elif rest.startswith("modulation.lin."):
-                out[f"{base}.adaLN_modulation.layers.1.{rest[15:]}"] = v
-            elif rest == "norm.query_norm.scale":
-                out[f"{base}.qk_norm.q_norm.weight"] = v
-            elif rest == "norm.key_norm.scale":
-                out[f"{base}.qk_norm.k_norm.weight"] = v
-            else:
-                raise KeyError(f"unrecognised FLUX key {key}")
-            continue
-        if key.startswith("img_in."):
-            leaf = key[7:]
-            out[f"x_embedder.proj.{leaf}"] = v.reshape(v.shape[0], 1, 1, v.shape[1]).contiguous() if leaf == "weight" else v
-        elif key.startswith("txt_in."):
-            out["context_embedder." + key[7:]] = v
-        elif key.startswith(("time_in.", "vector_in.")):
-            emb = "t_embedder" if key.startswith("time_in.") else "y_embedder"
-            _, layer, leaf = key.split(".")
-            out[f"{emb}.mlp.layers.{0 if layer == 'in_layer' else 2}.{leaf}"] = v
-        elif key.startswith("final_layer.adaLN_modulation.1."):
-            out["final_layer.adaLN_modulation.layers.1." + key.rsplit(".", 1)[1]] = v
-        elif key.startswith("final_layer.linear."):
-            out[key] = v
+            _, i, stream, j, qk = m.groups()
+            base = (f"multimodal_transformer_blocks.{i}.{_FLUX_STREAM[stream]}" if i is not None
+                    else f"unified_transformer_blocks.{j}.transformer_block")
+            out[f"{base}.qk_norm.{qk[0]}_norm.weight"] = v
         elif key.startswith("guidance_in."):
             continue  # quirk Q1: the reference ignores the guidance embedder (model_io.py:756,783)
         else:
@@ -133,26 +213,23 @@ def sd3_checkpoint_to_params(sd: Dict[str, Tensor], prefix: str = "model.diffusi
             continue
         if key.startswith(prefix):
             key = key[len(prefix):]
+        module, _, leaf = key.rpartition(".")
+        route = sd3_linear_route(module) if leaf in ("weight", "bias") else None
+        if route is not None:
+            _convert_linear(route, leaf, v, out, key)          # qkv: the k bias is dropped (model_io.py:389-390)
+            continue
         m = re.fullmatch(r"joint_blocks\.(\d+)\.(context_block|x_block)\.(.+)", key)
         if m:
             i, blk, rest = m.groups()
             stream = "text_transformer_block" if blk == "context_block" else "image_transformer_block"
             base = f"multimodal_transformer_blocks.{i}.{stream}"
-            if rest.startswith("attn.qkv."):
-                leaf = rest[9:]
-                for name, chunk in zip("qkv", v.chunk(3, dim=0)):
-                    if name == "k" and leaf == "bias":
-                        continue                     # model_io.py:389-390
-                    out[f"{base}.attn.{name}_proj.{leaf}"] = chunk.contiguous()
-            elif rest.startswith("attn.proj."):
-                out[f"{base}.attn.o_proj.{rest[10:]}"] = v
-            elif rest.startswith("attn.ln_q."):
+            if rest.startswith("attn.ln_q."):
                 out[f"{base}.qk_norm.q_norm.{rest[10:]}"] = v
             elif rest.startswith("attn.ln_k."):
                 out[f"{base}.qk_norm.k_norm.{rest[10:]}"] = v
             elif rest.startswith("adaLN_modulation."):
                 out[f"{base}.adaLN_modulation.layers.{rest[17:]}"] = v
-            else:                                    # mlp.fc1 / mlp.fc2 keep their names
+            else:                                    # any other block tensor keeps its name
                 out[f"{base}.{rest}"] = v
             continue
         if key == "pos_embed":

@@ -17,6 +17,9 @@ Differences that are deliberate (documented in DESIGN.md):
     every Euler step the latent cells outside the mask are reset to sigma_next * noise + (1 - sigma_next) * x_T
     (dk_inpaint_blend), and generate_image restores the pixels outside the mask from the input image in uint8
     (dk_image_post_masked).  A call without a mask launches exactly what it did before.
+  * LoRA extension (`load_lora` / `unload_lora`, lora.py; the reference has none): adapters keyed by the upstream
+    module names are merged in place into the packed MMDiT weights with dk_gemm's residual epilogue, so the denoise
+    loop runs the same kernels and captured graphs.  A pipeline without an adapter launches exactly what it did before.
 """
 from __future__ import annotations
 
@@ -376,6 +379,28 @@ class DiffusionPipeline:
             ep = {k: v.to(device=self.device, dtype=self.dtype) for k, v in ep.items()}
         self.encoder = VAEEncoder(ep, VAEEncoderConfig(), device=self.device)
         self._vae_encoder_params = None
+
+    # ------------------------------------------------------------------ LoRA adapters (an extension)
+    def load_lora(self, lora, scale: float = 1.0, name: Optional[str] = None):
+        """Merge a LoRA adapter into the MMDiT weights in place -> lora.LoraInfo(name, rank, n_targets, skipped).
+        `lora`: a .safetensors path or a dict str -> tensor, keyed by the upstream module names (BFL for FLUX, SAI for
+        SD3; PEFT lora_A / lora_B or kohya lora_unet_* lora_down / lora_up, optional .alpha).  `name` defaults to the
+        file stem ("lora<N>" for a dict); loading under an active name replaces that adapter, which is how its scale
+        is changed.  Every touched weight is W0 + sum_i scale_i * alpha_i / r_i * B_i @ A_i over the active adapters.
+        The merge runs on the device (one dk_gemm per weight); the denoise loop and its captured graphs are unchanged."""
+        from .lora import LoraMerger
+
+        if getattr(self, "_lora", None) is None:
+            self._lora = LoraMerger(self.mmdit)
+        return self._lora.load(lora, scale=scale, name=name)
+
+    def unload_lora(self, name: Optional[str] = None):
+        """Remove the adapter `name` (None: every adapter); weights no adapter touches any more are restored bit for
+        bit."""
+        if getattr(self, "_lora", None) is not None:
+            self._lora.unload(name)
+        elif name is not None:
+            raise KeyError(f"no active LoRA named {name!r} (active: [])")
 
     # ------------------------------------------------------------------ text (SURVEY.md §8 row f2)
     def load_text_encoders(self, clip_l=None, clip_g=None, t5=None, *, tokenizer_l=None, tokenizer_g=None,
